@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA kernels through the C-ABI)
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: the CPU implementation of the same cycle
+    python bench.py ... --dump-outputs DIR                   # also write one iteration's outputs (dump_outputs)
 
 BASELINE.json's metric is "train tokens/sec (GAN step)".  A "step" is one iteration of the reference's train loop
 (train.py:859-1090) on synthetic MAESTRO-vocab tokens: an MLE optimizer step of MemTransformerLM over the global batch
@@ -75,6 +76,9 @@ def parse():
     ap.add_argument("--cpu-batch", type=int, default=4)
     ap.add_argument("--warm-segments", type=int, default=None,
                     help="untimed MLE steps before timing (default: enough to fill the recurrence memory + capture graphs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU: after the timed steps, run each phase of the iteration from a fixed state and "
+                    "write what it computed (see dump_outputs) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -353,6 +357,10 @@ class Cycle:
                     trainable.append(prm)
             self.dfp = dp.FlatParams(trainable)
             self.dis_opt = dp.FusedClipAdam(self.dfp, lr, clip=WORK["clip"], world=world)
+        # --dump-outputs: the seeded initial parameters, the state dump_outputs() starts from
+        self.initial = None
+        if args.dump_outputs:
+            self.initial = [fp.flat.clone() for fp in (self.fp, self.dfp) if fp is not None]
         g = torch.Generator().manual_seed(dp.rank_seed(1111, rank))  # train.py:224
         pin = lambda t: t.pin_memory()
         nbuf = 4 * self.n_chunks
@@ -413,6 +421,80 @@ class Cycle:
         if self.gan and self.it % WORK["gan_freq"] == 0:
             self.gan_updates(e2e)
         self.it += 1
+
+
+def dump_outputs(cyc, out_dir, max_elems=1 << 20):
+    """Each phase of the timed iteration -- MLE step, discriminator update, generator update: forward + backward
+    through the same captured CUDA graphs, then the phase's fused clip + Adam step -- run from a state that is the same
+    in every run, written as float32 ``out_dir/<name>.npy``: ``mle_loss`` (per-token NLL [tgt_len, B]), ``mems`` (the
+    recurrence memory [n_layer+1, mem_len, B, d_model] it returns, flattened, batch chunks one after another),
+    ``dis_loss``, ``gp_loss``, ``gen_loss``, and per phase ``<mle|dis|gen>_grad`` (the gradient of the parameters the
+    phase's optimizer updates) and ``<mle|dis|gen>_update`` (parameters after the optimizer step minus before).  An
+    array of more than max_elems entries is written as a sample of its flat entries drawn from a fixed seed; at the
+    default workload the files come to about 27 MB.
+
+    The state: the seeded initial parameters, zero gradients, fresh optimizer moments, and a recurrence memory of
+    seeded N(0, 1) rows in the ring the timed steps left (same ring phase, so the captured graphs replay); it is
+    restored before every phase.  Not the state the timed steps leave: the fp32 gradient reductions are atomics, so
+    every step differs between runs in the last bits, and the ~50 optimizer steps and Gumbel sampling before the dump
+    grow that into a different trajectory.  From the fixed state only the phase's own reductions differ between runs.
+    The first Adam step moves a parameter by about lr * sign(gradient), so an entry whose gradient is at rounding level
+    can move by +-lr in one run and -+lr in the other.  profiles/dump_outputs_repeatability.txt compares two runs."""
+    import numpy as np
+    from tgan_b200.engine import notify_params_updated
+    inits = list(zip((cyc.fp, cyc.dfp), cyc.initial))
+
+    def restore():
+        for fp, init in inits:
+            fp.flat.copy_(init)
+            fp.zero_grad()
+        notify_params_updated()
+
+    arrays = {}
+
+    def optimizer_step(name, opt, init):
+        arrays[name + "_grad"] = opt.fp.grad.clone()
+        opt.m.zero_()
+        opt.v.zero_()
+        opt.steps = 0
+        opt.step()
+        arrays[name + "_update"] = opt.fp.flat - init
+        restore()
+
+    restore()
+    rng = torch.Generator(device=cyc.dev).manual_seed(1111)
+    d = WORK["d_model"]
+    for m in cyc.mems:
+        m.slabs[..., :d].normal_(0.0, 1.0, generator=rng)
+        m.slabs[..., d:].zero_()
+    losses = []
+    for c in range(cyc.n_chunks):  # Cycle.mle_step at iteration 0
+        ret = cyc.model(cyc.dev_data[c], cyc.dev_tgt[c], cyc.reset, "mle", cyc.mems[c])
+        losses.append(ret["mle"].detach())
+        cyc.mems[c] = ret["mems"]
+        (ret["mle"].mean() / cyc.n_chunks).backward()
+    arrays["mle_loss"] = torch.cat(losses, 1)
+    optimizer_step("mle", cyc.opt, cyc.initial[0])
+    if cyc.gan:  # Cycle.gan_updates at iteration 0
+        for j, (phase, opt, init) in enumerate((("dis_loss", cyc.dis_opt, cyc.initial[1]),
+                                                ("gen_loss", cyc.gen_opt, cyc.initial[0]))):
+            ret = cyc.model(cyc.dev_dis[j], None, None, phase)
+            arrays.update((k, v) for k, v in ret.items() if k in (phase, "gp_loss") and v is not None)
+            optimizer_step(phase[:3], opt, init)
+    torch.cuda.synchronize()
+    g = torch.Generator().manual_seed(0)
+
+    def sample(t, n=max_elems):
+        if t.numel() <= n:
+            return t
+        idx = torch.randint(0, t.numel(), (n,), generator=g).sort().values
+        return t.reshape(-1)[idx.to(t.device)]
+
+    # the memory materializes as fp32 (7.3 GB per chunk at the default workload): sample it chunk by chunk
+    arrays["mems"] = torch.cat([sample(m.materialize(), max_elems // len(cyc.mems)).reshape(-1) for m in cyc.mems])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), sample(t.detach()).float().cpu().numpy())
 
 
 def attention_roofline(dev, B, pk):
@@ -631,6 +713,9 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        # the dumped phases replay the captured MLE backward, whose bucket all-reduces no other rank would join
+        raise SystemExit("--dump-outputs runs on one GPU only (WORLD_SIZE=1)")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -689,6 +774,8 @@ def main():
     h2d, d2h = cyc.h2d / args.steps, cyc.d2h / args.steps
     torch.cuda.synchronize()
     final_loss = [float(x) for x in cyc.loss_host]
+    if args.dump_outputs:
+        dump_outputs(cyc, args.dump_outputs)
     global_batch = args.global_batch * world if args.scaling == "weak" else args.global_batch
     tokens = Q * global_batch * args.steps
     value = tokens / (ms_dev / 1e3)

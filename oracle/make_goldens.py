@@ -32,7 +32,9 @@ def token_stream(B, total_len, offset=0):
     return torch.from_numpy(np.stack(cols, 1))
 
 
-def run_mle_case(name, shape: O.TxlShape, seed, Q, B, nseg, reset_at=None, full_mems=True):
+def run_mle_case(name, shape: O.TxlShape, seed, Q, B, nseg, reset_at=None, full_mems=True, grad_thin=1):
+    """grad_thin: keep every grad_thin-th of the 2048 sampled entries of each large gradient (keeps the real-size
+    fixtures under 1 MB)."""
     params = O.init_params(shape, seed, dtype=torch.float64)
     model = ref_harness.build_reference_lm(shape, params, Q, dtype=torch.float64)
     for p in model.parameters():
@@ -73,7 +75,7 @@ def run_mle_case(name, shape: O.TxlShape, seed, Q, B, nseg, reset_at=None, full_
         if flat.numel() <= 4096:
             out["grad:" + key] = g.numpy()
         else:
-            idx = torch.linspace(0, flat.numel() - 1, 2048).long()
+            idx = torch.linspace(0, flat.numel() - 1, 2048).long()[::grad_thin]
             out["gidx:" + key] = idx.numpy()
             out["gval:" + key] = flat[idx].numpy()
     np.savez_compressed(os.path.join(GOLD, name + ".npz"), **out)
@@ -303,8 +305,10 @@ def main():
     cases = {
         "mle_tiny": lambda n: run_mle_case(n, tiny, seed=11, Q=8, B=3, nseg=4, reset_at=(2, 1)),
         "mle_tiny_samelen": lambda n: run_mle_case(n, tiny_sl, seed=12, Q=8, B=2, nseg=4, reset_at=(1, 0)),
-        "mle_real": lambda n: run_mle_case(n, real, seed=13, Q=16, B=2, nseg=3, reset_at=(2, 1), full_mems=False),
-        "mle_real_q32": lambda n: run_mle_case(n, real_q32, seed=18, Q=32, B=2, nseg=4, reset_at=(3, 1), full_mems=False),
+        "mle_real": lambda n: run_mle_case(n, real, seed=13, Q=16, B=2, nseg=3, reset_at=(2, 1), full_mems=False,
+                                           grad_thin=2),
+        "mle_real_q32": lambda n: run_mle_case(n, real_q32, seed=18, Q=32, B=2, nseg=4, reset_at=(3, 1), full_mems=False,
+                                               grad_thin=3),
         "generate_tiny": lambda n: run_generate_case(n, gen, seed=14, B=2, T=12, temperature=0.7),
         "gan_bert_tiny": lambda n: run_gan_case(n, gan, seed=15, B=3, dis_type="bert", loss_type="wgan-gp"),
         "gan_cnn_tiny": lambda n: run_gan_case(n, gan, seed=16, B=2, dis_type="cnn", loss_type="rsgan"),

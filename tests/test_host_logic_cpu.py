@@ -80,6 +80,16 @@ def test_reference_arm_prints_the_contract_line():
     assert "workload" in d["config"]
 
 
+def test_dump_outputs_is_refused_with_more_than_one_rank(tmp_path):
+    """The dump replays the captured MLE backward, which carries the bucket all-reduces: on one rank alone they would
+    wait for the others forever, so bench.py refuses before it touches a device."""
+    env = dict(os.environ, WORLD_SIZE="2", RANK="0", LOCAL_RANK="0")
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "2", "--dump-outputs",
+                          str(tmp_path / "dump")], capture_output=True, text=True, timeout=600, env=env)
+    assert out.returncode != 0 and "--dump-outputs runs on one GPU only" in out.stderr, out.stderr[-2000:]
+    assert not (tmp_path / "dump").exists()
+
+
 def test_lamb_chunk_table_covers_every_tensor_exactly_once():
     """FusedLamb cuts the flat parameter buffer into per-tensor chunks of <= 16384 elements (host logic, no kernel)."""
     import torch
