@@ -128,6 +128,19 @@ int tgan_relattn_fwd(int dtype, const void* q, int64_t ldq, const void* k, const
                      const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
                      void* out, int64_t ldo, float* lse, int B, int N, int Q, int M, int msl, int same_length,
                      float scale, float drop_p, uint64_t seed, uint64_t site, int impl, void* stream);
+/* Forward with a per-sequence key floor, for batches of left-padded prompts of different lengths (inference only: no
+ * backward honours the floor).  key_start: int32 [B], the absolute position of the first real token of sequence b;
+ * key_base: the absolute position of key row 0.  In addition to the mask above, key j of row i is masked iff
+ *     j < min(floor_b, i + M),   floor_b = max(reset[b] ? M : 0, key_start[b] - key_base)
+ * (the reset rule is the case key_start = NULL).  The clip at the row's own position i + M leaves a pad query row
+ * attending to itself only, so every output row is finite.  Relative attention depends on i - j only: a left-padded
+ * sequence then computes exactly what the same sequence without its pad rows computes.  key_start = NULL is exactly
+ * tgan_relattn_fwd.                                                                                          */
+int tgan_relattn_fwd_ragged(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
+                            const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
+                            void* out, int64_t ldo, float* lse, int B, int N, int Q, int M, int msl, int same_length,
+                            float scale, float drop_p, uint64_t seed, uint64_t site, int impl, void* stream,
+                            const int32_t* key_start, int64_t key_base);
 /* Backward.  dq [Q*B, ldq], dk, dv [K*B, lddkv] (dtype) and dr (fp32 [K, lddr]) are WRITTEN;
  * du, dvb (fp32 [N,64]) are ACCUMULATED (+=); delta is an fp32 scratch buffer of B*N*Q floats (row-wise dout.out) --
  * B*N*(M+1) floats when Q == 1: the fused single-token backward (csrc/relattn_decode.cu) keeps its dS row there.  */

@@ -208,6 +208,19 @@ __host__ __device__ __forceinline__ uint32_t dropout_thresh(float p) { return dr
 
 static inline int ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
+// Per-sequence key floor of the attention forward: floor_b = max(reset[b] ? M : 0, key_start[b] - key_base), clamped to
+// [0, K].  Query row i of sequence b masks the keys j < min(floor_b, i + M) (tgan_b200.h, tgan_relattn_fwd_ragged);
+// with key_start == NULL this is the reset rule, min(M, i + M) = M.  Computed once per sequence and CTA / warp.
+__device__ __forceinline__ int key_floor(const uint8_t* reset, const int32_t* key_start, int64_t key_base, int b, int M,
+                                         int K) {
+    int f = (reset && reset[b]) ? M : 0;
+    if (key_start) {
+        const int64_t s = (int64_t)key_start[b] - key_base;
+        f = max(f, (int)(s < 0 ? 0 : (s > K ? K : s)));
+    }
+    return f;
+}
+
 // ---- internal entry points shared between translation units ----------------------------------------------
 int tgan_gemm_simt(int dtype_ab, int dtype_c, int transA, int transB, int M, int N, int K, const void* A,
                    int64_t lda, const void* B, int64_t ldb, void* C, int64_t ldc, const float* bias, const void* aux,
@@ -218,10 +231,12 @@ int tgan_gemm_tc(int dtype_c, int transA, int transB, int M, int N, int K, const
                  const void* B, int64_t ldb, void* C, int64_t ldc, const float* bias, const void* aux,
                  int64_t ldaux, int flags, float alpha, float drop_p, uint64_t seed, uint64_t site, int force,
                  cudaStream_t st);
+// key_start / key_base: the per-sequence key floor (key_floor above); key_start = NULL switches it off
 int tgan_relattn_fwd_simt(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
-                          const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset, void* out,
-                          int64_t ldo, float* lse, int B, int N, int Q, int M, int msl, int same_length, float scale,
-                          float drop_p, uint64_t seed, uint64_t site, cudaStream_t st);
+                          const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
+                          const int32_t* key_start, int64_t key_base, void* out, int64_t ldo, float* lse, int B, int N,
+                          int Q, int M, int msl, int same_length, float scale, float drop_p, uint64_t seed, uint64_t site,
+                          cudaStream_t st);
 int tgan_relattn_bwd_simt(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
                           const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
                           const void* out, const void* dout, int64_t ldo, const float* lse, float* delta, void* dq,
@@ -231,8 +246,9 @@ int tgan_relattn_bwd_simt(int dtype, const void* q, int64_t ldq, const void* k, 
 // single-token (Q = 1) kernels (relattn_decode.cu); scratch = fp32 [B * N * (M + 1)]
 int tgan_relattn_fwd_decode1(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
                              const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
-                             void* out, int64_t ldo, float* lse, int B, int N, int M, int msl, int same_length, float scale,
-                             float drop_p, uint64_t seed, uint64_t site, cudaStream_t st);
+                             const int32_t* key_start, int64_t key_base, void* out, int64_t ldo, float* lse, int B, int N,
+                             int M, int msl, int same_length, float scale, float drop_p, uint64_t seed, uint64_t site,
+                             cudaStream_t st);
 int tgan_relattn_bwd_decode1(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
                              const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
                              const void* out, const void* dout, int64_t ldo, const float* lse, float* scratch, void* dq,
@@ -250,9 +266,9 @@ int tgan_bert_attn_jvp_mma(const void* qkv, int64_t ldq, const void* qkvd, int64
                            cudaStream_t st);
 // tcgen05 attention (bf16 only); return -1 when the shape is not eligible
 int tgan_relattn_fwd_tc(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* r,
-                        int64_t ldr, const float* u, const float* vb, const uint8_t* reset, void* out, int64_t ldo,
-                        float* lse, int B, int N, int Q, int M, int msl, int same_length, float scale, float drop_p,
-                        uint64_t seed, uint64_t site, cudaStream_t st);
+                        int64_t ldr, const float* u, const float* vb, const uint8_t* reset, const int32_t* key_start,
+                        int64_t key_base, void* out, int64_t ldo, float* lse, int B, int N, int Q, int M, int msl,
+                        int same_length, float scale, float drop_p, uint64_t seed, uint64_t site, cudaStream_t st);
 int tgan_relattn_bwd_tc(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* r,
                         int64_t ldr, const float* u, const float* vb, const uint8_t* reset, const void* out,
                         const void* dout, int64_t ldo, const float* lse, float* delta, void* dq, void* dk, void* dv,

@@ -31,6 +31,8 @@ struct DecArgs {
     float scale, scale_log2, drop_scale;
     uint32_t thresh, key;
     int split;               // backward: 1 = query side only (dk / dv of the memory rows are left to relattn_dec_keys)
+    const int32_t* key_start;  // forward: per-sequence key floor (common.cuh: key_floor), NULL = off
+    int64_t key_base;
 };
 
 // 8 consecutive elements kept in their storage format (bf16: one 16-byte register quad) until they are consumed: the
@@ -102,7 +104,8 @@ relattn_dec_fwd(const T* __restrict__ q, int64_t ldq, const T* __restrict__ k, c
 #pragma unroll
         for (int t = 0; t < 8; ++t) { qu[t] = x[t] + uu[t]; qv[t] = x[t] + vv[t]; }
     }
-    const int jlo = (reset && reset[b]) ? max(a.M, a.jlo0) : a.jlo0, jhi = a.K - 1;
+    // the key loop starts at the floor: masked rows (reset memory, the pad rows of a shorter prompt) are never streamed
+    const int jlo = max(a.jlo0, min(key_floor(reset, a.key_start, a.key_base, b, a.M, a.K), a.M)), jhi = a.K - 1;
     const uint32_t rowkey = attn_drop_rowkey(step_fold(a.key), (uint32_t)bn);
     float m = -INFINITY, l = 0.f, acc[8];
 #pragma unroll
@@ -456,6 +459,8 @@ DecArgs make_dec(int B, int N, int M, int msl, int same_length, float scale, flo
     a.drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
     a.thresh = drop_p > 0.f ? dropout_thresh16(drop_p) : 0u;
     a.key = dropout_key(seed, site);
+    a.key_start = nullptr;
+    a.key_base = 0;
     return a;
 }
 }  // namespace
@@ -465,9 +470,12 @@ int tgan_set_step_ctr_relattn_decode(const void* p) { return tgan_set_step_ctr_l
 // Eligibility: Q == 1, rows aligned for 16-byte (bf16) / 32-byte (fp32) vector access.
 int tgan_relattn_fwd_decode1(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
                              const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
-                             void* out, int64_t ldo, float* lse, int B, int N, int M, int msl, int same_length, float scale,
-                             float drop_p, uint64_t seed, uint64_t site, cudaStream_t st) {
+                             const int32_t* key_start, int64_t key_base, void* out, int64_t ldo, float* lse, int B, int N,
+                             int M, int msl, int same_length, float scale, float drop_p, uint64_t seed, uint64_t site,
+                             cudaStream_t st) {
     DecArgs a = make_dec(B, N, M, msl, same_length, scale, drop_p, seed, site);
+    a.key_start = key_start;
+    a.key_base = key_base;
     const int DW = N <= DW_MAX ? N : 4;
     const int grid = ceil_div((int64_t)B * N, DW);
     const size_t sm_f32 = (size_t)PF * 3 * DW * 32 * 32, sm_bf16 = (size_t)PF * 3 * DW * 32 * 16;

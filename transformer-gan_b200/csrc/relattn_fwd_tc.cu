@@ -59,6 +59,7 @@ struct FwdParams {
     float* lse;
     const float* u; const float* vb;
     const uint8_t* reset;
+    const int32_t* key_start; int64_t key_base;  // per-sequence key floor (NULL: off)
     int B, N, Q, M, K, msl, same_length;
     float scale_log2;  // scale * log2(e)
     float drop_scale; uint32_t drop_thresh; uint32_t drop_key;
@@ -79,23 +80,27 @@ relattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                    g_full = s_empty + 16, g_empty = g_full + 16, p_full = g_empty + 16, o_done = p_full + 16;
     const uint32_t sTmemPtr = o_done + 16;
     volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(gbase + (sTmemPtr - base));
+    // the key floor, parked next to the TMEM address: the row warps re-read it per tile instead of holding a register
+    volatile int* floor_sm = reinterpret_cast<volatile int*>(gbase + (sTmemPtr - base) + 4);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int bn = blockIdx.y, b = bn / p.N, n = bn % p.N;
     const int i0 = blockIdx.x * BQ;
     const int rows_here = min(BQ, p.Q - i0);
-    const bool reset_b = p.reset && p.reset[b];
+    // row i masks the keys j < min(floor_b, i + M): reset and the ragged-prompt key floor (common.cuh: key_floor)
+    const int floor_b = key_floor(p.reset, p.key_start, p.key_base, b, p.M, p.K);
 
     // key range needed by this query tile (CTA-uniform)
     int jlo = 0, jhi = min(p.K - 1, i0 + rows_here - 1 + p.M);
     if (p.same_length) jlo = max(0, i0 - p.msl + 1);
-    if (reset_b) jlo = max(jlo, p.M);
+    jlo = max(jlo, min(floor_b, i0 + p.M));
     const int t_lo = jlo / BJ, t_hi = jhi / BJ;
     const int nt = t_hi - t_lo + 1;      // >= 1
     const int nc = nt + NCHUNK - 1;      // G chunks
     const int P0 = p.Q - 1 - i0 - (BQ - 1) + BJ * t_lo;  // relative position of ring column 0
 
     if (threadIdx.x == 0) {
+        *floor_sm = floor_b;
         for (int s = 0; s < KV_STAGES; ++s) { mbar_init(kv_full + 8 * s, 1); mbar_init(kv_empty + 8 * s, 1); }
         for (int s = 0; s < R_STAGES; ++s) { mbar_init(r_full + 8 * s, 1); mbar_init(r_empty + 8 * s, 1); }
         for (int s = 0; s < 2; ++s) {
@@ -266,7 +271,7 @@ relattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
             float mx = -INFINITY;
             // CTA-uniform: a tile strictly inside every row's [lower, causal] window needs no per-element mask
             const bool interior = rows_here == BQ && j0 + BJ - 1 <= i0 + p.M &&
-                                  (!p.same_length || i0 + BQ - p.msl - j0 <= 0) && (!reset_b || p.M <= j0);
+                                  (!p.same_length || i0 + BQ - p.msl - j0 <= 0) && *floor_sm <= j0;
             if (interior) {
 #pragma unroll
                 for (int jj = 0; jj < BJ; ++jj) {
@@ -277,7 +282,7 @@ relattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                 int lim_hi = live ? (i + p.M - j0) : -1;  // jj <= lim_hi  (causal + memory)
                 int lim_lo = 0;                            // jj >= lim_lo
                 if (p.same_length) lim_lo = max(lim_lo, i - p.msl + 1 - j0);
-                if (reset_b) lim_lo = max(lim_lo, p.M - j0);
+                lim_lo = max(lim_lo, min(*floor_sm, i + p.M) - j0);
                 lim_hi = min(lim_hi, p.K - 1 - j0);
 #pragma unroll
                 for (int jj = 0; jj < BJ; ++jj) {
@@ -385,9 +390,9 @@ relattn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
 int tgan_set_step_ctr_relattn_fwd_tc(const void* p) { return tgan_set_step_ctr_local(p); }
 
 int tgan_relattn_fwd_tc(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* r,
-                        int64_t ldr, const float* u, const float* vb, const uint8_t* reset, void* out, int64_t ldo,
-                        float* lse, int B, int N, int Q, int M, int msl, int same_length, float scale, float drop_p,
-                        uint64_t seed, uint64_t site, cudaStream_t st) {
+                        int64_t ldr, const float* u, const float* vb, const uint8_t* reset, const int32_t* key_start,
+                        int64_t key_base, void* out, int64_t ldo, float* lse, int B, int N, int Q, int M, int msl,
+                        int same_length, float scale, float drop_p, uint64_t seed, uint64_t site, cudaStream_t st) {
     const int K = M + Q;
     const bool ok = Q >= 32 && (((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)r | (uintptr_t)out |
                                  (uintptr_t)u | (uintptr_t)vb) & 15) == 0;
@@ -405,6 +410,7 @@ int tgan_relattn_fwd_tc(const void* q, int64_t ldq, const void* k, const void* v
     if (rc) return rc;
     FwdParams p;
     p.q = (const bf16*)q; p.ldq = ldq; p.out = (bf16*)out; p.ldo = ldo; p.lse = lse; p.u = u; p.vb = vb; p.reset = reset;
+    p.key_start = key_start; p.key_base = key_base;
     p.B = B; p.N = N; p.Q = Q; p.M = M; p.K = K; p.msl = msl; p.same_length = same_length;
     p.scale_log2 = scale * 1.4426950408889634f;
     p.drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;

@@ -22,6 +22,8 @@ struct AttnArgs {
     float scale, drop_scale;
     uint32_t thresh;  // 16-bit threshold (0 = dropout off)
     uint32_t key;
+    const int32_t* key_start;  // forward only: per-sequence key floor (common.cuh: key_floor), NULL = off
+    int64_t key_base;
 };
 
 template <typename T>
@@ -85,7 +87,7 @@ relattn_fwd_simt(const T* __restrict__ q, int64_t ldq, const T* __restrict__ k, 
     __syncwarp();
     int jlo = 0, jhi = min(a.K - 1, i + a.M);
     if (a.same_length) jlo = max(0, i - a.msl + 1);
-    if (reset && reset[b]) jlo = max(jlo, a.M);
+    jlo = max(jlo, min(key_floor(reset, a.key_start, a.key_base, b, a.M, a.K), i + a.M));
     float m = -INFINITY, l = 0.f, acc[HS];
 #pragma unroll
     for (int d = 0; d < HS; ++d) acc[d] = 0.f;
@@ -158,7 +160,7 @@ relattn_fwd_decode(const T* __restrict__ q, int64_t ldq, const T* __restrict__ k
     __syncthreads();
     int jlo = 0, jhi = min(a.K - 1, i + a.M);
     if (a.same_length) jlo = max(0, i - a.msl + 1);
-    if (reset && reset[b]) jlo = max(jlo, a.M);
+    jlo = max(jlo, min(key_floor(reset, a.key_start, a.key_base, b, a.M, a.K), i + a.M));
     float m = -INFINITY, l = 0.f, acc0 = 0.f, acc1 = 0.f;  // m: warp-uniform running max; l: this lane's share of the sum
     for (int j0 = jlo + 32 * warp; j0 <= jhi; j0 += 32 * DECODE_WARPS) {
         const int j = j0 + lane;
@@ -528,20 +530,25 @@ AttnArgs make_args(int B, int N, int Q, int M, int msl, int same_length, float s
     a.drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
     a.thresh = drop_p > 0.f ? dropout_thresh16(drop_p) : 0u;
     a.key = dropout_key(seed, site);
+    a.key_start = nullptr;
+    a.key_base = 0;
     return a;
 }
 }  // namespace
 
 int tgan_relattn_fwd_simt(int dtype, const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv,
-                          const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset, void* out,
-                          int64_t ldo, float* lse, int B, int N, int Q, int M, int msl, int same_length, float scale,
-                          float drop_p, uint64_t seed, uint64_t site, cudaStream_t st) {
+                          const void* r, int64_t ldr, const float* u, const float* vb, const uint8_t* reset,
+                          const int32_t* key_start, int64_t key_base, void* out, int64_t ldo, float* lse, int B, int N,
+                          int Q, int M, int msl, int same_length, float scale, float drop_p, uint64_t seed, uint64_t site,
+                          cudaStream_t st) {
     AttnArgs a = make_args(B, N, Q, M, msl, same_length, scale, drop_p, seed, site);
+    a.key_start = key_start;
+    a.key_base = key_base;
     const bool vec_ok = ((((uintptr_t)k | (uintptr_t)v | (uintptr_t)r) & 31) == 0) && ldkv % 8 == 0 && ldr % 8 == 0;
     if (Q == 1 && vec_ok && ((((uintptr_t)q | (uintptr_t)out | (uintptr_t)u | (uintptr_t)vb) & 31) == 0) && ldq % 8 == 0 &&
         ldo % 8 == 0)
-        return tgan_relattn_fwd_decode1(dtype, q, ldq, k, v, ldkv, r, ldr, u, vb, reset, out, ldo, lse, B, N, M, msl,
-                                        same_length, scale, drop_p, seed, site, st);
+        return tgan_relattn_fwd_decode1(dtype, q, ldq, k, v, ldkv, r, ldr, u, vb, reset, key_start, key_base, out, ldo,
+                                        lse, B, N, M, msl, same_length, scale, drop_p, seed, site, st);
     if (Q <= DECODE_Q && vec_ok) {
         dim3 gd(Q, B * N);
         if (dtype == TGAN_F32)

@@ -101,9 +101,11 @@ class _TxlFunction(torch.autograd.Function):
     """One autograd node for the whole generator stack (embedding .. NLL or Gumbel-ST output)."""
 
     @staticmethod
-    def forward(ctx, model, mode, inp, target, reset, mems, temperature, noise, names, *params):
+    def forward(ctx, model, mode, inp, target, reset, mems, temperature, noise, names, grad_enabled, *params):
         eng = model._get_engine()
-        need_grad = any(ctx.needs_input_grad)  # grad mode is off inside Function.forward
+        # grad mode is off inside Function.forward, and needs_input_grad does not see a caller's no_grad(): that comes
+        # in as grad_enabled (a call under no_grad() records no graph, so nothing would ever read saved activations)
+        need_grad = grad_enabled and any(ctx.needs_input_grad)
         ectx = eng.forward(inp.detach(), reset, mems, mem_len=model.mem_len, same_length=model.same_length,
                            training=model.training, target=target if mode == "mle" else None,
                            n_pred=target.size(0) if mode == "mle" else None, save_for_backward=need_grad)
@@ -158,7 +160,7 @@ class _TxlFunction(torch.autograd.Function):
             dinp = torch.empty(ectx.Q * B, V, dtype=torch.float32, device=eng.device)
             L.convert(d, d.stride(0), dinp, V, ectx.Q * B, V, V)
             dinp = dinp.view(ectx.Q, B, V)
-        return (None, None, dinp, None, None, None, None, None, None) + (None,) * len(ctx.names)
+        return (None, None, dinp, None, None, None, None, None, None, None) + (None,) * len(ctx.names)
 
 
 class _GraphEntry:
@@ -382,6 +384,9 @@ class MemTransformerLM(nn.Module):
         if (self.use_cuda_graphs and mode == "mle" and isinstance(mems, RingMems) and self.mem_len > 0
                 and mems.length == self.mem_len and mems.bsz == data.shape[1] and torch.is_grad_enabled()
                 and self._graph_pending is None and data.dim() == 2):
+            if mems.key_start is not None:
+                raise L.TganError("a memory that carries a key floor (left-padded prompts) is for inference only: "
+                                  "it cannot enter a captured training step")
             ring = eng._prepare_ring(mems, data.shape[1], data.shape[0], self.mem_len)
             if ring is mems:  # steady state: the ring is reused in place, only (start, length) move
                 entry = self._graph_entry(eng, data, target, reset_mems, ring)
@@ -391,7 +396,7 @@ class MemTransformerLM(nn.Module):
                 ring.note_write((ring.start + ring.length) % ring.capacity, data.shape[0])  # the replay wrote the rows
                 return out, RingMems(ring.slabs, start, length, self.d_model, kv=ring.kv, shared=ring.shared)
         out = _TxlFunction.apply(self, mode, data, target, reset_mems, mems, temperature, noise, names,
-                                 *[pd[n] for n in names])
+                                 torch.is_grad_enabled(), *[pd[n] for n in names])
         return out, self._new_mems
 
     def forward(self, data, target, reset_mems, mems, status_vec=None):
@@ -417,7 +422,8 @@ class MemTransformerLM(nn.Module):
     # ---- batched generation (generate.py:207-304 for a whole batch, sampling on the device) ----------------
     @torch.no_grad()
     def generate_batched(self, start_ids, gen_len, *, technique="topk", topk=32, top_p=0.0, temperature=0.95,
-                         exclude_bos=True, empty_token=-1, num_empty_tokens_to_ignore=0, mems=None, uniforms=None):
+                         exclude_bos=True, empty_token=-1, num_empty_tokens_to_ignore=0, mems=None, uniforms=None,
+                         prompt_lengths=None):
         """The generation loop of generate.py:207-304 for ``B`` sequences at once with NO per-token host
         synchronisation: per step one single-token forward (projected-K/V cache, ``memory_length`` = ``self.mem_len``)
         and one ``tgan_sample_tokens`` launch (exclude-BOS, empty-bar suppression once the last
@@ -426,12 +432,23 @@ class MemTransformerLM(nn.Module):
 
         start_ids: int64 [T0, B] -- the conditioning tokens (unconditional generation: one row of BOS ids, :180-186).
         uniforms:  optional [gen_len, B] uniforms in [0, 1) replacing the device RNG (parity tests).
+        prompt_lengths: optional [B] ints -- prompts of different lengths: sequence b is primed with
+                   ``start_ids[:prompt_lengths[b], b]`` (right-padded input; the rows below are ignored).  Each
+                   sequence then generates exactly what it would generate alone.  The prompts are left-aligned on the
+                   device, and the returned memory carries a per-sequence key floor that hides the pad rows from
+                   every later call: ``generate_batched(ids[-1:], n, mems=mems)`` and ``forward_generate`` continue
+                   correctly (``mems.materialize()`` returns the pad rows too).  Needs ``mems=None``.  Such a memory
+                   is for inference only: it raises in any call that would train through it.
         Returns (ids int64 [gen_len, B], mems)."""
         eng = self._get_engine()
         dev = eng.device
         start_ids = start_ids.to(dev)
         T0, B = start_ids.shape
         mode = {"random": 0, "topk": 1, "nucleus": 2}[technique]
+        real = None  # [T0, B] bool: which rows of the (aligned) block are prompt tokens; None = all of them
+        if prompt_lengths is not None:
+            start_ids, real, mems = self._ragged_prompts(eng, start_ids, prompt_lengths, mems)
+            T0 = start_ids.shape[0]
         if T0 > 1:  # context pass over all but the last conditioning token (:190-199)
             _, mems = self._run("logits", start_ids[:-1], None, None, mems)
         cur = start_ids[-1:].contiguous()
@@ -441,8 +458,9 @@ class MemTransformerLM(nn.Module):
         if k > 0:
             # length of the run of `empty_token` at the end of each sequence (conditioning tokens included, :235-238)
             run = torch.zeros(B, dtype=torch.int32, device=dev)
-            for t in range(T0):
-                run = torch.where(start_ids[t] == empty_token, run + 1, torch.zeros_like(run))
+            for t in range(T0):  # (pad rows precede a sequence's prompt: they leave the run at 0)
+                hit = start_ids[t] == empty_token if real is None else (start_ids[t] == empty_token) & real[t]
+                run = torch.where(hit, run + 1, torch.zeros_like(run))
         V = self.n_token
         for t in range(gen_len):
             ectx = eng.forward(cur, None, mems, mem_len=self.mem_len, same_length=self.same_length, training=False,
@@ -459,3 +477,23 @@ class MemTransformerLM(nn.Module):
             if k > 0:
                 run = torch.where(out[t] == empty_token, run + 1, torch.zeros_like(run))
         return out, mems
+
+    def _ragged_prompts(self, eng, start_ids, prompt_lengths, mems):
+        """Right-padded prompts [T0, B] of lengths len_b -> (the prompts left-aligned into [max len_b, B], which rows
+        of it are real, an empty ring whose key floor starts sequence b at its first real row)."""
+        T0, B = start_ids.shape
+        if mems is not None:
+            raise ValueError("prompt_lengths needs mems=None: pad rows inside an existing memory cannot be masked")
+        lens = torch.as_tensor(prompt_lengths).to("cpu", torch.int64).reshape(-1)
+        if lens.numel() != B:
+            raise ValueError(f"prompt_lengths has {lens.numel()} entries for a batch of {B}")
+        if bool((lens < 1).any()) or bool((lens > T0).any()):
+            raise ValueError(f"prompt_lengths must lie in [1, {T0}] (the rows of start_ids)")
+        T = int(lens.max())
+        pad = (T - lens).to(start_ids.device)
+        rows = torch.arange(T, device=start_ids.device).view(T, 1)
+        # row t of column b holds prompt token t - pad_b; the pad rows repeat token 0 (any valid id: they are masked)
+        aligned = start_ids.gather(0, (rows - pad).clamp(min=0))
+        ring = eng.new_ring(B, max(T - 1, 1), self.mem_len)
+        ring.key_start = pad.to(torch.int32)
+        return aligned, rows >= pad, ring

@@ -68,14 +68,22 @@ class RingMems:
 
     ``start`` is the ring position of logical memory row 0, ``length`` the number of valid memory rows.
     The reference returns a fresh ``[n_layer+1, M, B, d_model]`` fp32 tensor per call; ``materialize()``
-    produces exactly that tensor (for tests, checkpoints and the generate.py self-check)."""
+    produces exactly that tensor (for tests, checkpoints and the generate.py self-check).
+
+    A ring that holds left-padded prompts of different lengths (``generate_batched(prompt_lengths=...)``) carries a
+    per-sequence key floor: ``key_start`` (device int32 [B]) is the absolute position of the first real row of each
+    sequence and ``pos0`` the absolute position of logical memory row 0; every forward over the ring masks the keys
+    below the floor (tgan_relattn_fwd_ragged).  ``key_start`` is None for every other ring.  Such a ring is for
+    inference only: a forward that saves activations for a backward raises."""
 
     def __init__(self, slabs: torch.Tensor, start: int, length: int, d_model: int, kv: Optional[dict] = None,
-                 shared: Optional[dict] = None):
+                 shared: Optional[dict] = None, key_start: Optional[torch.Tensor] = None, pos0: int = 0):
         self.slabs = slabs
         self.start = start
         self.length = length
         self.d_model = d_model
+        self.key_start = key_start  # shared by every window over the same slabs, like ``kv``
+        self.pos0 = pos0
         # State shared by every window (handle) over the same slabs: ``gen`` counts the writes into the ring and
         # ``writes`` logs the most recent ones as (gen, position, count).  A handle remembers the generation it was
         # produced at; it stays valid until a LATER write lands inside its window (the reference returns fresh
@@ -133,7 +141,8 @@ class RingMems:
         return out
 
     def materialize(self) -> torch.Tensor:
-        """-> fp32 [n_layer+1, length, B, d_model] (logical order), via tgan_convert."""
+        """-> fp32 [n_layer+1, length, B, d_model] (logical order), via tgan_convert.  Every row, the pad rows below
+        a ``key_start`` floor included: row m of sequence b is real iff pos0 + m >= key_start[b]."""
         S, C, B, DP = self.slabs.shape
         out = torch.empty(S, self.length, B, self.d_model, dtype=torch.float32, device=self.slabs.device)
         for s in range(S):
@@ -481,6 +490,7 @@ class TxlEngine:
             new.kv.update(buf=nb, lo=0, hi=n, tag=self.pack_epoch)
         new.length = n
         new.gen = new.shared["gen"]
+        new.key_start, new.pos0 = ring.key_start, ring.pos0  # logical row 0 stays row 0
         return new
 
     # -- forward ------------------------------------------------------------------------------------------
@@ -491,6 +501,10 @@ class TxlEngine:
         ``nll`` (fp32 [T*B], when target is given), ``logits`` (fp32 [T*B, VP]) and ``new_mems``."""
         d, lay, dt = self.d, self.layout, self.dtype
         DP, NH, DIP, VP, D = d.DP, d.NH, d.DIP, d.VP, d.d_model
+        if save_for_backward and getattr(mems, "key_start", None) is not None:
+            # no backward kernel honours the key floor: the gradients would include the pad rows
+            raise L.TganError("a memory that carries a key floor (left-padded prompts) is for inference only: "
+                              "it cannot be used in a forward that saves activations for a backward")
         self.pack()
         Q, B = inp.shape[0], inp.shape[1]
         ring = self._prepare_ring(mems, B, Q, mem_len) if mem_len > 0 else self.new_ring(B, Q, 0)
@@ -608,7 +622,7 @@ class TxlEngine:
             lse = self._buf(B * d.n_head * Q, dtype=torch.float32)
             L.relattn_fwd(q, kv, kv, 2 * NH, r, self._v("u"), self._v("vb"), reset_u8, att, lse, B, d.n_head, Q, M, msl,
                           same_length, scale, p_att, seed, self._site(cid, 8 + 4 * l), impl=self.impl, k_off=kv_off,
-                          v_off=kv_off + NH)
+                          v_off=kv_off + NH, key_start=ring.key_start, key_base=ring.pos0)
             # O projection + dropout + residual (fp32) -> LN
             ooff, old = self._m(p + "Wo")
             z1 = self._buf(R, DP, dtype=torch.float32)
@@ -670,7 +684,8 @@ class TxlEngine:
         if mem_len > 0:
             new_len = min(M + Q, mem_len)
             new_start = (ring.start + M + Q - new_len) % C
-            ctx.new_mems = RingMems(ring.slabs, new_start, new_len, D, kv=ring.kv, shared=ring.shared)
+            ctx.new_mems = RingMems(ring.slabs, new_start, new_len, D, kv=ring.kv, shared=ring.shared,
+                                    key_start=ring.key_start, pos0=ring.pos0 + M + Q - new_len)
         else:
             ctx.new_mems = None
         return ctx

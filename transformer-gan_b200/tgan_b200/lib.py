@@ -46,6 +46,7 @@ _SIGS = {
     "tgan_ln_bwd": [I, P, L, P, L, P, P, P, P, L, P, L, P, P, P, I, I, I, F, U, U, P],
     "tgan_dropout": [I, P, L, P, L, I, I, F, U, U, P],
     "tgan_relattn_fwd": [I, P, L, P, P, L, P, L, P, P, P, P, L, P, I, I, I, I, I, I, F, F, U, U, I, P],
+    "tgan_relattn_fwd_ragged": [I, P, L, P, P, L, P, L, P, P, P, P, L, P, I, I, I, I, I, I, F, F, U, U, I, P, P, L],
     "tgan_relattn_bwd": [I, P, L, P, P, L, P, L, P, P, P, P, P, L, P, P, P, P, P, L, P, L, P, P, I, I, I, I, I, I,
                          F, F, U, U, I, P],
     "tgan_relattn_bwd_step": [I, I, P, L, P, P, L, P, L, P, P, P, P, P, L, P, P, P, P, P, L, P, L, P, P, I, I, I, I, I,
@@ -278,12 +279,19 @@ def dropout(src, dst, rows, cols, lds, ldd, p, seed, site, src_off=0, dst_off=0)
 
 
 def relattn_fwd(q, k, v, ldkv, r, u, vb, reset, out, lse, B, N, Q, M, msl, same_length, scale, drop_p, seed, site,
-                impl=IMPL_AUTO, k_off=0, v_off=0):
+                impl=IMPL_AUTO, k_off=0, v_off=0, key_start=None, key_base=0):
+    """key_start (int32 [B]) / key_base: the per-sequence key floor of tgan_relattn_fwd_ragged (left-padded prompts);
+    key_start=None calls tgan_relattn_fwd."""
     es = q.element_size()
-    _call("tgan_relattn_fwd", dtype_code(q.dtype), q.data_ptr(), q.stride(0), k.data_ptr() + k_off * es,
-          v.data_ptr() + v_off * es, ldkv, r.data_ptr(), r.stride(0), _ptr(u), _ptr(vb), _ptr(reset),
-          out.data_ptr(), out.stride(0), _ptr(lse), B, N, Q, M, msl, int(same_length), scale, drop_p, seed,
-          site, impl, _stream())
+    args = (dtype_code(q.dtype), q.data_ptr(), q.stride(0), k.data_ptr() + k_off * es, v.data_ptr() + v_off * es, ldkv,
+            r.data_ptr(), r.stride(0), _ptr(u), _ptr(vb), _ptr(reset), out.data_ptr(), out.stride(0), _ptr(lse), B, N, Q,
+            M, msl, int(same_length), scale, drop_p, seed, site, impl, _stream())
+    if key_start is None:
+        _call("tgan_relattn_fwd", *args)
+    else:
+        if key_start.dtype != torch.int32 or key_start.numel() != B:
+            raise TganError("relattn_fwd: key_start must be an int32 tensor of B entries")
+        _call("tgan_relattn_fwd_ragged", *args, key_start.data_ptr(), int(key_base))
 
 
 def relattn_bwd(q, k, v, ldkv, r, u, vb, reset, out, dout, lse, delta, dq, dk, dv, lddkv, dr, du, dvb, B, N, Q, M,
