@@ -52,3 +52,16 @@ def test_product_path_never_imports_the_oracle():
             if f.endswith(".py"):
                 txt = open(os.path.join(dirpath, f)).read()
                 assert "txl_oracle" not in txt and "ref_harness" not in txt and "import oracle" not in txt, f
+
+
+def test_library_has_no_environment_or_build_switches():
+    """The kernels a call runs depend only on its arguments: no environment variable read by the library or its
+    binding, and no project macro that compiles a second variant of a kernel."""
+    pkg = os.path.join(ROOT, "transformer-gan_b200")
+    csrc = os.path.join(pkg, "csrc")
+    for f in sorted(os.listdir(csrc)):
+        if f.endswith((".cu", ".cuh")):
+            txt = open(os.path.join(csrc, f)).read()
+            assert "getenv(" not in txt, f
+            assert not re.search(r"#\s*if(n?def|\s+defined)\W*TGAN_", txt), f
+    assert "os.environ" not in open(os.path.join(pkg, "tgan_b200", "lib.py")).read()

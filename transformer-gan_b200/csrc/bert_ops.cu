@@ -10,8 +10,6 @@
 // embeddings) theta sits behind the encoder, so that derivative is J_enc applied to a direction = one JVP pass; no
 // double-backward graph is ever built.  The dense layers run on tgan_gemm (tcgen05); everything here is HBM- or
 // latency-bound glue plus the 64 x 64 attention tiles (3 % of the encoder's FLOPs).
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace {
@@ -446,8 +444,7 @@ extern "C" int tgan_ln_jvp(int dtype, const float* zd, int64_t ldzd, const float
 
 // bf16 tiles with d_head a multiple of 16 and 16-byte aligned rows run on the tensor cores (bert_attn_mma.cu)
 static bool mma_ok(int dtype, int dh, int64_t ld0, int64_t ld1, int64_t ld2, const void* p0, const void* p1, const void* p2) {
-    static const bool off = getenv("TGAN_BERT_ATTN_SIMT") != nullptr;
-    return !off && dtype == TGAN_BF16 && dh % 16 == 0 && ld0 % 8 == 0 && ld1 % 8 == 0 && ld2 % 8 == 0 &&
+    return dtype == TGAN_BF16 && dh % 16 == 0 && ld0 % 8 == 0 && ld1 % 8 == 0 && ld2 % 8 == 0 &&
            ((((uintptr_t)p0 | (uintptr_t)p1 | (uintptr_t)p2) & 15) == 0);
 }
 

@@ -13,7 +13,6 @@
 // Operand layouts: K-major (row-major [rows, K]) or MN-major (row-major [K, rows]); both are read by TMA with
 // the same 64 x 64-element swizzled boxes and described to the tensor core through the UMMA descriptors.
 // Used for every dense contraction of the path: QKV / R / O projections, FFN, logits, and all dgrad / wgrad.
-#include <stdlib.h>
 #include <string.h>
 
 #include "tc_common.cuh"
@@ -113,17 +112,6 @@ constexpr int EPI_BIAS_VEC = 1 << 22; // internal: bias pointer is 16-byte align
 constexpr int EPI_TMA = 1 << 23;      // internal: C leaves through shared memory + TMA store (reduce-add for ACCUM / split-K)
 constexpr int EPI_ALPHA = 1 << 24;    // internal: alpha != 1
 constexpr int STAGE_BYTES = 32 * 128; // one epilogue warp's staging box: 32 rows x 128 bytes, 128-byte swizzle
-
-#ifdef TGAN_PROFILE
-__device__ long long g_gemm_prof[32];
-#define GPROF_DECL long long _pt = clock64(); long long _acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#define GPROF(i) { const long long _n = clock64(); _acc[i] += _n - _pt; _pt = _n; }
-#define GPROF_DUMP(base) if (blockIdx.x == 1 && lane == 0) { for (int _i = 0; _i < 8; ++_i) g_gemm_prof[(base) + _i] = _acc[_i]; }
-#else
-#define GPROF_DECL
-#define GPROF(i)
-#define GPROF_DUMP(base)
-#endif
 
 template <int BN> struct Cfg {
     static constexpr int STAGES = BN == 256 ? 4 : 6;
@@ -362,14 +350,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (warp == 0) {
         // ===================== TMA producer =====================
         if (lane == 0) {
-            GPROF_DECL
             int s = 0; uint32_t ph = 0;
             for (int w = blockIdx.x; w < num_work; w += gridDim.x) {
                 const Work wk = get_work<BN>(w, num_tiles, tiles_n, nk, kb_per_split);
                 for (int kb = wk.kb0; kb < wk.kb1; ++kb) {
-                    GPROF(0)
                     mbar_wait(empty0 + 8 * s, ph ^ 1);
-                    GPROF(1)
                     const uint32_t fb = full0 + 8 * s;
                     mbar_expect_tx(fb, A_BYTES + B_BYTES);
                     const uint32_t a_dst = sA + s * A_BYTES, b_dst = sB + s * B_BYTES;
@@ -386,8 +371,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     if (++s == STAGES) { s = 0; ph ^= 1; }
                 }
             }
-            GPROF(0)
-            GPROF_DUMP(0)
         }
     } else if (warp == 1) {
         // ===================== MMA issuer =====================
@@ -398,19 +381,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const uint64_t db0 = B_MN ? umma_smem_desc(sB, 8192, 1024) : umma_smem_desc(sB, 16, 1024);
         constexpr uint32_t a_kstep = (A_MN ? 2048 : 32) >> 4, b_kstep = (B_MN ? 2048 : 32) >> 4;
         int s = 0; uint32_t ph = 0; int it = 0;
-        GPROF_DECL
         for (int w = blockIdx.x; w < num_work; w += gridDim.x, ++it) {
             const Work wk = get_work<BN>(w, num_tiles, tiles_n, nk, kb_per_split);
             const int as = it & 1; const uint32_t aph = (it >> 1) & 1;
-            GPROF(0)
             mbar_wait(tempty0 + 8 * as, aph ^ 1);
-            GPROF(1)
             tcgen05_fence_after();
             const uint32_t d_tmem = tmem_base + as * BN;
             for (int kb = wk.kb0; kb < wk.kb1; ++kb) {
-                GPROF(0)
                 mbar_wait(full0 + 8 * s, ph);
-                GPROF(2)
                 tcgen05_fence_after();
                 if (elect_one()) {
                     const uint64_t da = da0 + (uint64_t)((s * A_BYTES) >> 4), db = db0 + (uint64_t)((s * B_BYTES) >> 4);
@@ -424,8 +402,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 if (++s == STAGES) { s = 0; ph ^= 1; }
             }
         }
-        GPROF(0)
-        GPROF_DUMP(8)
     } else {
         // ===================== epilogue warps =====================
         // warp w may only touch TMEM lanes 32*(w%4) .. +31; the two warps sharing a lane quarter split the columns.
@@ -440,13 +416,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const uint32_t stage_u32 = sStage + (warp - 2) * STAGE_BYTES;
         bool pending = false;  // a bulk store issued by this warp may still be reading the staging box
         int it = 0;
-        GPROF_DECL
         for (int w = blockIdx.x; w < num_work; w += gridDim.x, ++it) {
             const Work wk = get_work<BN>(w, num_tiles, tiles_n, nk, kb_per_split);
             const int as = it & 1; const uint32_t aph = (it >> 1) & 1;
-            GPROF(0)
             mbar_wait(tfull0 + 8 * as, aph);
-            GPROF(1)
             tcgen05_fence_after();
             const int row0 = wk.m0 + 32 * eq;
             const int64_t row = row0 + lane;
@@ -459,18 +432,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         const int c0 = b0 + 32 * seg;
                         if (wk.n0 + c0 >= N) break;  // warp-uniform; the rest of the box is clipped by the tensor map
                         uint32_t regs[32];
-                        GPROF(0)
                         tmem_ld32(tmem_base + as * BN + c0 + ((uint32_t)(32 * eq) << 16), regs);
                         tmem_ld_wait();
-                        GPROF(2)
                         if (seg == 0 && pending) {
                             if (lane == 0) tma_store_wait_read();
                             __syncwarp();
                             pending = false;
                         }
-                        GPROF(3)
                         if (row < M) epi_row32_smem<TC, EPI>(regs, row, lane, wk.n0 + c0, seg, N, stage, ldc, ep, dkey);
-                        GPROF(4)
                     }
                     fence_proxy_async_smem();
                     __syncwarp();
@@ -480,19 +449,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         tma_store_commit();
                     }
                     pending = true;
-                    GPROF(5)
                 }
             } else if constexpr (EPI < 0) {
 #pragma unroll 1
                 for (int c0 = eh * (BN / 2); c0 < (eh + 1) * (BN / 2); c0 += 32) {
                     if (wk.n0 + c0 >= N) break;  // warp-uniform
                     uint32_t regs[32];
-                    GPROF(0)
                     tmem_ld32(tmem_base + as * BN + c0 + ((uint32_t)(32 * eq) << 16), regs);
                     tmem_ld_wait();
-                    GPROF(2)
                     if (row < M) epi_row32<TC>(regs, row, wk.n0 + c0, N, C, ldc, ep, dkey);
-                    GPROF(4)
                 }
             }
             tcgen05_fence_before();
@@ -500,8 +465,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (lane == 0) mbar_arrive(tempty0 + 8 * as);
         }
         if (pending && lane == 0) tma_store_wait_all();
-        GPROF(0)
-        if (warp == 2) { GPROF_DUMP(16) }
     }
     tcgen05_fence_before();
     __syncthreads();
@@ -798,11 +761,6 @@ int launch_layout(int transA, int transB, int epi_ct, const CUtensorMap& tmA, co
 
 extern "C" int tgan_has_tcgen05(void) { return 1; }
 int tgan_set_step_ctr_gemm_tc(const void* p) { return tgan_set_step_ctr_local(p); }
-#ifdef TGAN_PROFILE
-extern "C" int tgan_debug_gemm_prof(long long* host32) {
-    return (int)cudaMemcpyFromSymbol(host32, g_gemm_prof, sizeof(long long) * 32);
-}
-#endif
 
 int tgan_gemm_tc(int dtype_c, int transA, int transB, int M, int N, int K, const void* A, int64_t lda, const void* B,
                  int64_t ldb, void* C, int64_t ldc, const float* bias, const void* aux, int64_t ldaux, int flags,
@@ -872,7 +830,7 @@ int tgan_gemm_tc(int dtype_c, int transA, int transB, int M, int N, int K, const
     CUtensorMap tmC;
     memset(&tmC, 0, sizeof(tmC));
     const bool accum = (ep.flags & (TGAN_EPI_ACCUM | EPI_ATOMIC)) != 0;
-    if (vec && ((int64_t)N * esz_c) % 16 == 0 && !(accum && dtype_c != TGAN_F32) && !getenv("TGAN_GEMM_NO_TMA_EPI")) {
+    if (vec && ((int64_t)N * esz_c) % 16 == 0 && !(accum && dtype_c != TGAN_F32)) {
         rc = tc::make_tmap_2d_dt(&tmC, C, (uint64_t)M, (uint64_t)N, (uint64_t)ldc, 32, dtype_c == TGAN_F32 ? 32 : 64,
                                  dtype_c == TGAN_F32);
         if (rc) return rc;
@@ -885,13 +843,11 @@ int tgan_gemm_tc(int dtype_c, int transA, int transB, int M, int N, int K, const
         ep.flags = (ep.flags & ~TGAN_EPI_ACCUM) | EPI_ATOMIC;
     // compile-time epilogue variant: whole 8-column groups, aligned bias, bf16 aux
     int epi_ct = -1;
-    if ((ep.flags & EPI_TMA) && N % 8 == 0 && !ep.aux_is_f32 && (!(ep.flags & TGAN_EPI_BIAS) || (ep.flags & EPI_BIAS_VEC)) &&
-        !getenv("TGAN_GEMM_NO_CT_EPI"))
+    if ((ep.flags & EPI_TMA) && N % 8 == 0 && !ep.aux_is_f32 && (!(ep.flags & TGAN_EPI_BIAS) || (ep.flags & EPI_BIAS_VEC)))
         epi_ct = (ep.flags & (TGAN_EPI_BIAS | TGAN_EPI_RELU | TGAN_EPI_MASK_POS | TGAN_EPI_ADD_AUX | TGAN_EPI_DROPOUT)) |
                  (alpha != 1.0f ? EPI_ALPHA : 0);
     // 2-CTA pairs for the nn.Linear layout when there are enough 256 x 256 tiles to fill the 74 pairs
-    static const int use_2cta = getenv("TGAN_GEMM_2CTA") ? atoi(getenv("TGAN_GEMM_2CTA")) : 1;
-    if (use_2cta && !transA && transB && epi_ct >= 0 && splits == 1 && M >= 2048 &&
+    if (!transA && transB && epi_ct >= 0 && splits == 1 && M >= 2048 &&
         ceil_div(M, 256) * ceil_div(N, 256) >= sm_count() / 2) {
         CUtensorMap tmA2, tmB2;
         rc = tc::make_tmap_2d(&tmA2, A, (uint64_t)M, (uint64_t)K, (uint64_t)lda, 128, BK);

@@ -1,10 +1,10 @@
 // tcgen05 relative-position attention BACKWARD for sm_100a (bf16 operands, fp32 accumulation in TMEM).
 // Reference: autograd of mem_transformer.py:201-244 (+ _rel_shift :133-147, mask :495-547); SURVEY.md section 9.
 //
-// One CTA per (b, n); requires Q <= 128 (one query tile) so dK / dV tiles are complete per CTA.  4*SPLIT + 8 warps:
-//   row warps   (4*SPLIT of them) thread = (query row = TMEM lane, column slice): warp w owns lane quarter w & 3 and
-//               the CW = 64/SPLIT-column slice w >> 2 of every 64-wide tile, so each query row is served by SPLIT
-//               threads.  They do ONLY the per-score work: G ring, P, dS, publish.
+// One CTA per (b, n); requires Q <= 128 (one query tile) so dK / dV tiles are complete per CTA.  16 warps:
+//   row warps   (8 of them) thread = (query row = TMEM lane, column half): warp w owns lane quarter w & 3 and the
+//               32-column half w >> 2 of every 64-wide tile, so each query row is served by 2 threads.  They do
+//               ONLY the per-score work: G ring, P, dS, publish.
 //   drain warps (4, one per TMEM lane quarter): move the finished key-side results out of tensor memory -- dK / dV
 //               tiles (scaled, bf16, staged for the TMA store) and dR chunks (red.global.add over the batch).  In
 //               round 1 the row warps did this between their own phases: 37 % of their tile time (profiles/
@@ -36,16 +36,13 @@ constexpr int HS = TGAN_HS;  // 64
 constexpr int BQ = 128;      // query rows per CTA
 constexpr int BJ = 64;       // keys per tile
 constexpr int RING_COLS = 192;
-#ifndef TGAN_BWD_SPLIT
-#define TGAN_BWD_SPLIT 2
-#endif
-constexpr int SPLIT = TGAN_BWD_SPLIT;   // threads per query row (2 or 4): each owns CW columns of every 64-wide tile
+constexpr int SPLIT = 2;   // threads per query row: each owns CW columns of every 64-wide tile
 constexpr int CW = BJ / SPLIT;
+static_assert(CW == 32, "a thread's column slice is one tmem_ld32");
 constexpr int ROW_WARPS = 4 * SPLIT;
 constexpr int DRAIN0 = ROW_WARPS;          // drain warps DRAIN0 .. DRAIN0 + 3 (DRAIN0 % 4 == 0: warp w reads lane quarter w & 3)
 constexpr int MMA_WARP = ROW_WARPS + 4;
 constexpr int NTHREADS = 32 * (ROW_WARPS + 8);
-static_assert(SPLIT == 2 || SPLIT == 4, "row split");
 
 constexpr int B_OFF_QU = 0;
 constexpr int B_OFF_QV = B_OFF_QU + 16384;
@@ -81,31 +78,12 @@ struct BwdParams {
     float drop_scale; uint32_t drop_thresh; uint32_t drop_key;
 };
 
-#ifdef TGAN_PROFILE
-__device__ long long g_bwd_prof[16];
-#define PROF_DECL long long _pt = clock64(); long long _acc[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-#define PROF(i) { const long long _n = clock64(); _acc[i] += _n - _pt; _pt = _n; }
-#define PROF_DUMP() if (blockIdx.x == 200 && threadIdx.x == 0) { for (int _i = 0; _i < 16; ++_i) g_bwd_prof[_i] = _acc[_i]; }
-__device__ long long g_bwd_prof_mma[16];
-#define PROF_DUMP_MMA() if (blockIdx.x == 200) { for (int _i = 0; _i < 13; ++_i) g_bwd_prof_mma[_i] = _acc[_i]; }
-#else
-#define PROF_DECL
-#define PROF(i)
-#define PROF_DUMP()
-#define PROF_DUMP_MMA()
-#endif
-
 __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
-// the SPLIT warps serving one lane quarter (w, w + 4, ...) meet on named barrier 1 + quarter
+// the two warps serving one lane quarter (w, w + 4) meet on named barrier 1 + quarter
 __device__ __forceinline__ void pair_sync(int quarter) {
     asm volatile("bar.sync %0, %1;" ::"r"(quarter + 1), "n"(32 * SPLIT) : "memory");
-}
-// CW consecutive fp32 TMEM columns of this thread's lane
-__device__ __forceinline__ void tmem_ld_cw(uint32_t taddr, uint32_t* r) {
-    if constexpr (CW == 32) tmem_ld32(taddr, r);
-    else tmem_ld16(taddr, r);
 }
 
 __global__ void __launch_bounds__(NTHREADS, 1)
@@ -113,7 +91,6 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                       const __grid_constant__ CUtensorMap tmR, const __grid_constant__ CUtensorMap tmDK,
                       const __grid_constant__ CUtensorMap tmDV, BwdParams p) {
     extern __shared__ uint8_t smem_raw[];
-    PROF_DECL
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t* gbase = smem_raw + (base - smem_u32(smem_raw));
     const uint32_t sQu = base + B_OFF_QU, sQv = base + B_OFF_QV, sDO = base + B_OFF_DO, sK = base + B_OFF_K,
@@ -220,7 +197,6 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
 #pragma unroll
         for (int t = 0; t < SPLIT; ++t) delta += delta_x[t];
     }
-    PROF(0)
 
     if (warp == MMA_WARP + 1) {
         // =========================== K / V producer ===========================
@@ -272,14 +248,10 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                        n_qv = umma_smem_desc(sQv, 8192, 1024), n_k0 = umma_smem_desc(sK, 8192, 1024),
                        n_rd = umma_smem_desc(sRD, 8192, 1024);
         const uint64_t ring_mn0 = umma_smem_desc_noswz(sDR, 128, DR_GROUP), ring_k0 = umma_smem_desc_noswz(sDR, DR_GROUP, 128);
-        PROF(0)
         auto mma_s = [&](int tt) {
             if (tt >= nt) return;
-            PROF(0)
             mbar_wait(k_full + 8 * (tt & 1), (tt >> 1) & 1);
-            PROF(1)
             mbar_wait(s_empty, (tt & 1) ^ 1);
-            PROF(2)
             tcgen05_fence_after();
             if (elect_one()) {
                 const uint64_t dk = k_k0 + (uint64_t)(((tt & 1) * 8192) >> 4);
@@ -291,11 +263,8 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
         };
         auto mma_dp = [&](int tt) {
             if (tt >= nt) return;
-            PROF(0)
             mbar_wait(v_full, tt & 1);
-            PROF(3)
             mbar_wait(dp_empty, (tt & 1) ^ 1);
-            PROF(4)
             tcgen05_fence_after();
             if (elect_one()) {
 #pragma unroll
@@ -307,11 +276,8 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
         };
         auto mma_g = [&](int cc) {
             if (cc >= nc) return;
-            PROF(0)
             mbar_wait(rg_full + 8 * (cc & 1), (cc >> 1) & 1);
-            PROF(5)
             mbar_wait(g_empty, (cc & 1) ^ 1);
-            PROF(6)
             tcgen05_fence_after();
             if (elect_one()) {
                 const uint64_t dr = k_rg0 + (uint64_t)(((cc & 1) * 8192) >> 4);
@@ -323,9 +289,7 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
             __syncwarp();
         };
         auto mma_key = [&](int tt) {
-            PROF(0)
             mbar_wait(p_full, tt & 1);
-            PROF(7)
             if (tt > 0) mbar_wait(kd_empty, (tt - 1) & 1);  // dK / dV of tile tt-1 have left tensor memory
             tcgen05_fence_after();
             if (elect_one()) {
@@ -345,11 +309,8 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
             __syncwarp();
         };
         auto mma_rel = [&](int cc) {
-            PROF(0)
             mbar_wait(rd_full, cc & 1);
-            PROF(8)
             if (cc > 0) mbar_wait(dr_empty, (cc - 1) & 1);  // the row warps have drained dR of chunk cc-1
-            PROF(9)
             tcgen05_fence_after();
             if (elect_one()) {
                 const uint32_t cboff = ((cc % 3) * (BJ * 16)) >> 4;  // chunk cc = ring positions 64*(cc%3) .. +63
@@ -375,8 +336,6 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
         for (int cc = nt; cc < nc; ++cc) mma_rel(cc);
         if (elect_one()) umma_commit(fin);
         __syncwarp();
-        PROF(0)
-        if (lane == 0) { PROF_DUMP_MMA() }
     } else if (warp >= DRAIN0) {
         // =========================== drain warps: key-side results out of tensor memory ===========================
         // dK / dV of tile tk and dR of chunk cc sit in TMEM in the M = 64 layout: row r = 16 * quarter + lane, lanes 0..15.
@@ -461,7 +420,7 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                 mbar_wait(g_full, consumed & 1);
                 tcgen05_fence_after();
                 uint32_t g[CW];
-                tmem_ld_cw(tmem_base + TB_G + hc + lane_off, g);
+                tmem_ld32(tmem_base + TB_G + hc + lane_off, g);
                 tmem_ld_wait();
                 tcgen05_fence_before();
                 __syncwarp();
@@ -471,9 +430,7 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                 for (int c = 0; c < CW; ++c) dst[c * BQ] = __float2half_rn(__uint_as_float(g[c]));
                 ++consumed;
             }
-            PROF(1)
             pair_sync(quarter);  // A: both halves of the new chunk are in the ring
-            PROF(2)
             const int j0 = (t_lo + tt) * BJ;
             const int start = (BQ - 1 - ii + BJ * tt + hc) % RING_COLS;  // ring column of this thread's jj = 0
             const int wrap = RING_COLS - start;                         // first jj that wraps around
@@ -485,12 +442,11 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                 mbar_wait(s_full, tt & 1);
                 tcgen05_fence_after();
                 uint32_t sr[CW];
-                tmem_ld_cw(tmem_base + TB_S + hc + lane_off, sr);
+                tmem_ld32(tmem_base + TB_S + hc + lane_off, sr);
                 tmem_ld_wait();
                 tcgen05_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(s_empty);
-                PROF(3)
                 const bool interior = rows_here == BQ && j0 + BJ - 1 <= p.M && (!p.same_length || BQ - p.msl - j0 <= 0) &&
                                       (!reset_b || p.M <= j0);
                 if (interior) {
@@ -513,20 +469,16 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                     }
                 }
             }
-            PROF(4)
             pair_sync(quarter);  // B: both threads of the row are done reading the G ring for this tile
-            PROF(5)
             // 3. dP
             mbar_wait(dp_full, tt & 1);
             tcgen05_fence_after();
             uint32_t dpr[CW];
-            tmem_ld_cw(tmem_base + TB_DP + hc + lane_off, dpr);
+            tmem_ld32(tmem_base + TB_DP + hc + lane_off, dpr);
             tmem_ld_wait();
             tcgen05_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(dp_empty);
-            PROF(6)
-            PROF(8)
             // 4. P~ = keep(P), dS = P (keep(dP) - delta), packed to bf16 pairs in registers
             uint32_t ptw[CW / 2], dsw[CW / 2];
             {
@@ -551,10 +503,8 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
             // 5. the ring third this tile's scatter is about to reuse must have been consumed (dqR / dR MMAs of chunk
             //    tt-1), and the P~ buffer must be free again (the drain warps staged tile tt-1's dK / dV in it and the
             //    TMA store has finished reading them)
-            PROF(7)
             if (tt > 0) {
                 mbar_wait(rdone, (tt - 1) & 1);
-                PROF(9)
                 mbar_wait(ks_empty, (tt - 1) & 1);
             }
             if (tt + 2 >= nt) {
@@ -585,7 +535,6 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
             fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) mbar_arrive(p_full);
-            PROF(10)
         }
         // dq = (dqK + dqR) / sqrt(d); du / dvb = column sums over the query rows.  `fin` is committed after the last
         // MMA (a parity wait on `rdone` would be ambiguous here: the row warps are up to three phases behind it).
@@ -593,8 +542,8 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
         tcgen05_fence_after();
         {
             uint32_t a[CW], c2[CW];
-            tmem_ld_cw(tmem_base + TB_DQK + hc + lane_off, a);
-            tmem_ld_cw(tmem_base + TB_DQR + hc + lane_off, c2);
+            tmem_ld32(tmem_base + TB_DQK + hc + lane_off, a);
+            tmem_ld32(tmem_base + TB_DQR + hc + lane_off, c2);
             tmem_ld_wait();
             tcgen05_fence_before();
             if (live) {
@@ -619,8 +568,6 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
                 atomicAdd(&p.dvb[n * HS + hc + lane], sv * p.scale);
             }
         }
-        PROF(11)
-        PROF_DUMP()
     }
     tcgen05_fence_before();
     __syncthreads();
@@ -630,13 +577,6 @@ relattn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
     }
 }
 }  // namespace
-
-#ifdef TGAN_PROFILE
-extern "C" int tgan_debug_bwd_prof(long long* host16) {
-    cudaMemcpyFromSymbol(host16 + 16, g_bwd_prof_mma, sizeof(long long) * 16);
-    return (int)cudaMemcpyFromSymbol(host16, g_bwd_prof, sizeof(long long) * 16);
-}
-#endif
 
 int tgan_set_step_ctr_relattn_bwd_tc(const void* p) { return tgan_set_step_ctr_local(p); }
 

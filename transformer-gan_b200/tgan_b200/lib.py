@@ -17,7 +17,7 @@ EPI_BIAS, EPI_RELU, EPI_MASK_POS, EPI_ADD_AUX, EPI_ACCUM, EPI_DROPOUT, EPI_AUX_F
 IMPL_AUTO, IMPL_SIMT, IMPL_TC = 0, 1, 2
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("TGAN_B200_LIB", os.path.join(_HERE, "libtgan_b200.so"))  # override: instrumented builds
+LIB_PATH = os.path.join(_HERE, "libtgan_b200.so")
 
 
 class TganError(RuntimeError):
