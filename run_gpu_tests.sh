@@ -12,4 +12,5 @@ done
 run gemm_tc_epi tests/test_kernels_gpu.py -k "gemm_epilogues and (cdtype0-2 or cdtype1-2)"
 run gemm_tc_big tests/test_kernels_gpu.py -k "large_k or cta_pair"
 run relattn tests/test_relattn_gpu.py
+run bert_attn tests/test_bert_attn_gpu.py
 run model tests/test_model_gpu.py

@@ -4,7 +4,21 @@ import math
 import pytest
 import torch
 
+import dropmask as DM
+from attn_readout import attn_readout
+
 pytestmark = pytest.mark.gpu
+
+
+@pytest.fixture(autouse=True)
+def _no_step_counter():
+    """The host dropout masks assume no step counter; an earlier test may have registered the process-wide one."""
+    with DM.pinned_step_counter(None):
+        yield
+
+
+def _keep(seed, site, rows, cols, ld, p, step=None):
+    return torch.from_numpy(DM.elem_keep(seed, site, rows, cols, ld, p, step)).cuda()
 
 
 def _lib():
@@ -69,15 +83,16 @@ def test_gemm_epilogues(impl, cdtype):
     assert (got - torch.where(aux.float() > 0, 2.0 * ref0, torch.zeros_like(ref0))).abs().max() < tol * 8
     C0 = _rand(M, N, dtype=cdtype, seed=8)
     assert (run(L.EPI_ACCUM, C0=C0) - (ref0 + C0.float())).abs().max() < tol * 4
-    # dropout: same mask from both implementations (counter hash), right keep rate, survivors scaled by 1/(1-p)
-    d = run(L.EPI_DROPOUT, drop_p=0.25, seed=11, site=5)
-    keep = d != 0
-    assert abs(keep.float().mean().item() - 0.75) < 0.01
-    assert ((d - ref0 / 0.75).abs() * keep).max() < tol * 6
-    C2 = torch.zeros(M, N, device="cuda", dtype=cdtype)
-    L.gemm(A, B, C2, M=M, N=N, K=K, flags=L.EPI_DROPOUT, drop_p=0.25, seed=11, site=5, impl=3 - impl)
-    torch.cuda.synchronize()
-    assert torch.equal(C2 != 0, keep), "SIMT and tcgen05 epilogues disagree on the dropout mask"
+    # dropout: the host mask at element row * ldc + col, survivors scaled by 1/(1-p); also with a row pitch wider than N
+    for ldc in (N, N + 24):
+        C = torch.full((M, ldc), 7.0, device="cuda", dtype=cdtype)
+        L.gemm(A, B, C, M=M, N=N, K=K, ldc=ldc, flags=L.EPI_DROPOUT, drop_p=0.25, seed=2 ** 35 + 11, site=5, impl=impl)
+        torch.cuda.synchronize()
+        keep, d = _keep(2 ** 35 + 11, 5, M, N, ldc, 0.25), C[:, :N].float()
+        assert torch.all(d[~keep] == 0), "an element the mask drops survived"
+        assert torch.all(d[keep & (ref0.abs() > 1)] != 0), "an element the mask keeps was dropped"
+        assert ((d - ref0 / 0.75).abs() * keep).max() < tol * 6
+        assert torch.all(C[:, N:] == 7.0)
 
 
 def test_gemm_tc_large_k_accumulation_and_persistence():
@@ -106,7 +121,7 @@ def test_gemm_tc_large_k_accumulation_and_persistence():
 @pytest.mark.parametrize("cdtype", [torch.bfloat16, torch.float32])
 def test_gemm_tc_cta_pair_kernel(cdtype):
     """Shapes with >= 74 output tiles of 256 x 256 take the 2-CTA (cta_group::2) kernel: plain, fused FFN and residual
-    epilogues, ragged M / N edges, dropout mask identical to the SIMT kernel's."""
+    epilogues, ragged M / N edges, and the dropout mask the host regenerates."""
     L = _lib()
     M, N, K = 4100, 1288, 520
     A, B = _rand(M, K, dtype=torch.bfloat16, seed=3, scale=0.5), _rand(N, K, dtype=torch.bfloat16, seed=4, scale=0.5)
@@ -124,9 +139,10 @@ def test_gemm_tc_cta_pair_kernel(cdtype):
     assert (run(L.EPI_BIAS | L.EPI_RELU) - torch.relu(ref0 + bias)).abs().max() < tol
     assert (run(L.EPI_ADD_AUX) - (ref0 + aux.float())).abs().max() < tol
     d = run(L.EPI_BIAS | L.EPI_RELU | L.EPI_DROPOUT, drop_p=0.25, seed=11, site=5)
-    d1 = run(L.EPI_BIAS | L.EPI_RELU | L.EPI_DROPOUT, impl=1, drop_p=0.25, seed=11, site=5)
-    pos = torch.relu(ref0 + bias) > 0.05
-    assert torch.equal((d != 0) & pos, (d1 != 0) & pos), "2-CTA and SIMT epilogues disagree on the dropout mask"
+    keep, want = _keep(11, 5, M, N, N, 0.25), torch.relu(ref0 + bias) / 0.75
+    assert torch.all(d[~keep] == 0), "an element the mask drops survived"
+    assert torch.all(d[keep & (want > 0.5)] != 0), "an element the mask keeps was dropped"
+    assert ((d - want).abs() * keep).max() < tol / 0.75
 
 
 def test_gemm_fp32_simt_exact():
@@ -173,15 +189,11 @@ def test_layernorm_fwd_bwd(dtype):
     assert (dz[:, :D].double() - zr.grad).abs().max() < (1e-4 if dtype == torch.float32 else 3e-2)
     assert (dg[:D].double() - gref.grad).abs().max() < (1e-3 if dtype == torch.float32 else 0.2)
     assert (db[:D].double() - bref.grad).abs().max() < (1e-3 if dtype == torch.float32 else 0.2)
-    keep = dzd[:, :D] != 0
-    assert abs(keep.float().mean().item() - 0.8) < 0.02
+    # dz_drop: the host mask at element row * DP + col
+    keep = _keep(3, 9, rows, D, DP, 0.2)
+    assert torch.all(dzd[:, :D][~keep] == 0)
+    assert torch.all(dzd[:, :D][keep & (dz[:, :D].abs() > 1e-3)] != 0)
     assert ((dzd[:, :D].float() - dz[:, :D].float() / 0.8).abs() * keep).max() < 3e-2
-    # the mask equals the one tgan_dropout / the GEMM epilogue generate for the same (seed, site, ld)
-    ones = torch.ones(rows, DP, device="cuda", dtype=dtype)
-    m2 = torch.empty_like(ones)
-    L.dropout(ones, m2, rows, DP, DP, DP, 0.2, 3, 9)
-    nz = dz[:, :D] != 0
-    assert torch.equal((m2[:, :D] != 0) & nz, keep & nz)
 
 
 def test_embedding_and_posemb():
@@ -209,6 +221,74 @@ def test_embedding_and_posemb():
     assert (pe[:, :D].cpu() - ref).abs().max() < 2e-4  # fp32 sin/cos of arguments up to 1151 rad
     L.pos_emb(inv, pe, K, D, DP, 100, 0.0, 0, 0)
     assert (pe[:, :D].cpu() - O.positional_embedding(K, D, 100)).abs().max() < 2e-4
+
+
+@pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
+def test_elementwise_dropout_sites_match_host_mask(dtype):
+    """tgan_dropout, embed_fwd, embed_bwd and pos_emb with dropout on: exactly the host mask at row * ld + col."""
+    L = _lib()
+    p, seed, site = 0.1, 2 ** 33 + 5, 2 ** 32 + 7
+    rows, cols, lds, ldd = 301, 200, 216, 232
+    src = _rand(rows, lds, dtype=dtype, seed=3)
+    dst = torch.full((rows, ldd), 9.0, device="cuda", dtype=dtype)
+    L.dropout(src, dst, rows, cols, lds, ldd, p, seed, site)
+    keep = _keep(seed, site, rows, cols, ldd, p)
+    want = torch.where(keep, src[:, :cols].float() / (1 - p), torch.zeros(()).cuda())
+    tol = 1e-6 if dtype == torch.float32 else 1e-2
+    assert ((dst[:, :cols].float() - want).abs() <= tol * want.abs()).all()
+    assert torch.all(dst[:, cols:] == 9.0)
+
+    V, D, DP, n = 310, 500, 512, 257
+    E = torch.zeros(320, DP, device="cuda", dtype=dtype)
+    E[:V, :D] = _rand(V, D, seed=1, dtype=dtype)
+    ids = torch.randint(0, V, (n,), device="cuda")
+    out = torch.empty(n, DP, device="cuda", dtype=dtype)
+    L.embed_fwd(ids, E, out, n, D, DP, math.sqrt(D), p, seed, site)
+    keep = _keep(seed, site, n, D, DP, p)
+    want = torch.where(keep, E[ids, :D].float() * (math.sqrt(D) / (1 - p)), torch.zeros(()).cuda())
+    assert ((out[:, :D].float() - want).abs() <= 1e-5 + tol * want.abs()).all()
+    assert torch.all(out[:, D:] == 0)
+
+    dout = _rand(n, DP, dtype=dtype, seed=2)
+    dE = torch.zeros(320, DP, device="cuda")
+    L.embed_bwd(ids, dout, dE, n, V, D, DP, math.sqrt(D), p, seed, site)
+    ref = torch.zeros(V, D, device="cuda", dtype=torch.float64)
+    ref.index_add_(0, ids, dout[:, :D].double() * keep * (math.sqrt(D) / (1 - p)))
+    assert (dE[:V, :D].double() - ref).abs().max() < 1e-3
+
+    K = 300
+    pe = torch.empty(K, DP, device="cuda", dtype=dtype)
+    pe0 = torch.empty(K, DP, device="cuda", dtype=dtype)
+    inv = (1 / (10000 ** (torch.arange(0.0, D, 2.0) / D))).cuda()
+    L.pos_emb(inv, pe0, K, D, DP, -1, 0.0, 0, 0)
+    L.pos_emb(inv, pe, K, D, DP, -1, p, seed, site)
+    keep = _keep(seed, site, K, D, DP, p)
+    want = torch.where(keep, pe0[:, :D].float() / (1 - p), torch.zeros(()).cuda())
+    assert ((pe[:, :D].float() - want).abs() <= 1e-6 + tol * want.abs()).all()
+    assert torch.all(pe[:, D:] == 0)
+
+
+def test_step_counter_folds_into_the_masks():
+    """With a registered step counter every mask key becomes mix32(key ^ counter * 0x9E3779B1) (common.cuh step_fold):
+    an element-wise mask and an attention mask follow the host port with the same counter value, and differ from the
+    masks without it."""
+    L = _lib()
+    rows, cols, p = 64, 256, 0.25
+    ones = torch.ones(rows, cols, device="cuda")
+    with DM.pinned_step_counter(977):
+        m = torch.empty_like(ones)
+        L.dropout(ones, m, rows, cols, cols, cols, p, 5, 6)
+        torch.cuda.synchronize()
+        assert torch.equal(m != 0, _keep(5, 6, rows, cols, cols, p, step=977))
+        assert not torch.equal(m != 0, _keep(5, 6, rows, cols, cols, p))
+        attn_readout(16, 30, torch.float32, 1, False, p, 7, 8, step=977)
+    # on exit the process-wide counter (if one was created) is registered again
+    ctr = L._step_counters.get(torch.cuda.current_device())
+    m0 = torch.empty_like(ones)
+    L.dropout(ones, m0, rows, cols, cols, cols, p, 5, 6)
+    torch.cuda.synchronize()
+    step = None if ctr is None else int(ctr.item())
+    assert torch.equal(m0 != 0, _keep(5, 6, rows, cols, cols, p, step=step))
 
 
 def test_cross_entropy_and_gumbel():

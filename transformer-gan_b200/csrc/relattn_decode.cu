@@ -356,9 +356,14 @@ relattn_dec_bwd(const T* __restrict__ q, int64_t ldq, const T* __restrict__ k, c
     // them over the batch on the side stream.
     if (active && kg == 0) {
         if constexpr (SPLIT) {
+            // scalar stores: the rows start 2 * N * K * B floats into the scratch, which is only 8-byte aligned when
+            // N * K * B is odd (an odd head count, batch and key count)
             float* rows = dsbuf + 2 * (int64_t)a.N * a.K * a.B + (int64_t)b * a.N * HS + col;
-            store8(rows, dqk);
-            store8(rows + (int64_t)a.B * a.N * HS, dqr);
+#pragma unroll
+            for (int t = 0; t < 8; ++t) {
+                rows[t] = dqk[t];
+                rows[t + (int64_t)a.B * a.N * HS] = dqr[t];
+            }
         } else {
 #pragma unroll
             for (int t = 0; t < 8; ++t) {
