@@ -252,6 +252,21 @@ int tgan_bert_attn_jvp(int dtype, const void* qkv, int64_t ldq, const void* qkvd
 int tgan_sample_tokens(const float* logits, int64_t ldl, const float* u, const uint8_t* suppress_empty, int64_t* ids,
                        float* probs_out, int64_t ldp, int rows, int V, int exclude_bos, int empty_token, int mode,
                        int topk, float top_p, float temperature, uint64_t seed, uint64_t site, void* stream);
+/* One step of generation from a request queue (MemTransformerLM.generate_requests): column b of logits [B, ldl]
+ * serves request req[b] (-1 = idle), with that request's settings req_i int32 [R][5] = (mode, topk, exclude_bos,
+ * empty_token, num_empty_tokens_to_ignore) and req_f fp32 [R][2] = (temperature, top_p), validated by the caller.
+ * cur int64 [B] holds the column's input token of this step; run int32 [B] is the length of the run of empty_token
+ * at the end of the column's inputs: reset where start[b] == step (a request starts), then extended by cur[b].  The
+ * empty token is suppressed once run >= num_empty_tokens_to_ignore > 0.  The draw is tgan_sample_tokens' exact
+ * arithmetic, on u[out_off[b]] (u != NULL and out_off[b] >= 0) or on Philox keyed by (seed, site, b).  The sample
+ * goes to out[out_off[b]] when out_off[b] >= 0, and cur[b] becomes the next step's input: forced_next[b] when it
+ * is >= 0, else the sample (forced_next = NULL: the sample; an idle column keeps its input).  req, start, out_off,
+ * forced_next: int32 [B], the step's rows of the host schedule.  probs_out (optional, fp32 [B, ldp]): the filtered,
+ * renormalised distribution of every busy column.                                                            */
+int tgan_sample_step(const float* logits, int64_t ldl, const int32_t* req, const int32_t* start,
+                     const int32_t* out_off, const int32_t* forced_next, const int32_t* req_i, const float* req_f,
+                     const float* u, int32_t* run, int64_t* cur, int64_t* out, float* probs_out, int64_t ldp, int B,
+                     int V, int step, uint64_t seed, uint64_t site, void* stream);
 
 /* ---- data-parallel gradient all-reduce (SURVEY 8e): replaces DistributedDataParallel's implicit all-reduce,
  * train.py:649-655 / :904.  The library binds libnccl.so.2 at run time (tgan_nccl_load, optional explicit path).

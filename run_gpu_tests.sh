@@ -14,3 +14,4 @@ run gemm_tc_big tests/test_kernels_gpu.py -k "large_k or cta_pair"
 run relattn tests/test_relattn_gpu.py
 run bert_attn tests/test_bert_attn_gpu.py
 run model tests/test_model_gpu.py
+run requests tests/test_generate_requests_gpu.py

@@ -8,8 +8,11 @@ the reference -- ``MemTransformerLM(cfg, n_token, vec_len)`` with ``forward(data
 CPU fallback: calling the model on a CPU tensor raises.
 """
 import contextlib
+import heapq
 import os
 import weakref
+from dataclasses import dataclass
+from typing import List, NamedTuple
 
 import torch
 import torch.nn as nn
@@ -224,6 +227,87 @@ class _TxlGraphFunction(torch.autograd.Function):
         torch._foreach_add_(grads, staged)  # one multi-tensor kernel: .grad += this segment's gradients
         model._graph_pending = None
         return (None, None, None) + (None,) * len(ctx.names)
+
+
+# ---- generation from a request queue: host schedule --------------------------------------------------------
+_TECHNIQUES = {"random": 0, "topk": 1, "nucleus": 2}
+
+
+@dataclass
+class GenRequest:
+    """One prime to continue with ``MemTransformerLM.generate_requests``; the settings mirror ``generate_batched``'s
+    keywords.  prompt: int64 [T], T >= 1 (the conditioning tokens); gen_len >= 1 tokens are generated."""
+    prompt: torch.Tensor
+    gen_len: int
+    technique: str = "topk"
+    topk: int = 32
+    top_p: float = 0.0
+    temperature: float = 0.95
+    exclude_bos: bool = True
+    empty_token: int = -1
+    num_empty_tokens_to_ignore: int = 0
+
+
+class RequestSchedule(NamedTuple):
+    """The step-by-column plan of ``generate_requests``.  ``tables`` int32 [4, S, B] holds, per step t and column b:
+    forced   -- the input token of the step, or -1 for "the column's sample of step t - 1";
+    req      -- the request served, or -1 for an idle column;
+    out_off  -- where the step's sample goes in the flat output, or -1 when it is not kept;
+    key_start -- the step at which the column's current request started (an idle column: t itself).
+    The row written at step t has absolute position t, so key_start is also the request's key floor.
+    ``out_base[r]``: offset of request r's first generated token in the flat output."""
+    tables: torch.Tensor
+    out_base: List[int]
+
+    @property
+    def forced(self):
+        return self.tables[0]
+
+    @property
+    def req(self):
+        return self.tables[1]
+
+    @property
+    def out_off(self):
+        return self.tables[2]
+
+    @property
+    def key_start(self):
+        return self.tables[3]
+
+
+def request_schedule(prompts, gen_lens, batch_size) -> RequestSchedule:
+    """Plan ``len(prompts)`` requests on min(batch_size, len(prompts)) columns.  Request r occupies one column for
+    T_r + gen_len_r - 1 consecutive steps: it feeds its T_r prompt tokens one per step, the step that feeds the last
+    one samples its first token, and each later step feeds the previous sample.  Requests go in list order to the
+    column that frees first, ties to the lowest column.  Idle columns (the tail of the queue) are fed token 0 and floored
+    at their own row: they produce nothing.  prompts: 1-D int sequences (CPU); gen_lens: ints >= 1."""
+    B = min(batch_size, len(prompts))
+    free = [(0, c) for c in range(B)]  # (step at which the column frees, column): a heap
+    place = []
+    for prompt, g in zip(prompts, gen_lens):
+        t0, c = heapq.heappop(free)
+        place.append((t0, c))
+        heapq.heappush(free, (t0 + len(prompt) + g - 1, c))
+    S = max(t for t, _ in free)
+    tables = torch.empty(4, S, B, dtype=torch.int32)
+    forced, req, out_off, key_start = tables
+    forced.zero_()
+    req.fill_(-1)
+    out_off.fill_(-1)
+    key_start.copy_(torch.arange(S, dtype=torch.int32).view(S, 1).expand(S, B))
+    out_base, base = [], 0
+    for r, ((t0, c), prompt, g) in enumerate(zip(place, prompts, gen_lens)):
+        T = len(prompt)
+        n = T + g - 1
+        forced[t0:t0 + T, c] = torch.as_tensor(prompt, dtype=torch.int32)
+        forced[t0 + T:t0 + n, c] = -1
+        req[t0:t0 + n, c] = r
+        out_off[t0 + T - 1:t0 + n, c] = torch.arange(base, base + g, dtype=torch.int32)
+        key_start[t0:t0 + n, c] = t0
+        out_base.append(base)
+        base += g
+    return RequestSchedule(tables, out_base)
 
 
 class MemTransformerLM(nn.Module):
@@ -497,3 +581,83 @@ class MemTransformerLM(nn.Module):
         ring = eng.new_ring(B, max(T - 1, 1), self.mem_len)
         ring.key_start = pad.to(torch.int32)
         return aligned, rows >= pad, ring
+
+    @torch.no_grad()
+    def generate_requests(self, requests, batch_size, *, uniforms=None):
+        """Continue every ``GenRequest`` of a queue, ``batch_size`` sequences at a time: a column that finishes a request
+        takes the next one at the following step (``request_schedule``), so no column waits for the longest sequence
+        of a fixed batch.  Prompts are fed one token per step.  All columns share one ring memory; each column carries
+        a per-sequence key floor raised to the step at which its current request started, so a request never sees the
+        rows of the requests before it and computes what it computes alone.  Per step: the single-token forward of
+        ``generate_batched`` and one ``tgan_sample_step`` launch (per-request settings, empty-bar run, sampling, next
+        input), with no host synchronisation: the schedule is uploaded once, up front.
+
+        Request r's tokens equal ``generate_batched(prompt[:, None], gen_len, <its settings>, uniforms=u[:, None])``
+        up to rounding.  With ``same_length=False`` that holds for prompts of up to mem_len + 2 tokens: a longer prompt
+        row sees at most mem_len earlier rows here, as every single-token step does, while generate_batched's context
+        pass lets it see the whole prompt.
+
+        requests: list of GenRequest.  uniforms: optional list with one [gen_len_r] tensor of uniforms in [0, 1) per
+        request, replacing the device RNG (parity tests).  Returns a list whose entry r is request r's generated ids,
+        int64 [gen_len_r] on the model's device (views into one buffer)."""
+        reqs = list(requests)
+        if not reqs:
+            raise ValueError("generate_requests needs at least one request")
+        if int(batch_size) < 1:
+            raise ValueError(f"batch_size must be >= 1, got {batch_size}")
+        if self.mem_len <= 0:
+            raise ValueError("generate_requests needs mem_len > 0: the requests of a column share its ring memory")
+        V = self.n_token
+        prompts, gen_lens, rows_i, rows_f = [], [], [], []
+        for r, q in enumerate(reqs):
+            p = torch.as_tensor(q.prompt).cpu()
+            if p.dim() != 1 or p.numel() < 1 or p.dtype.is_floating_point or p.dtype == torch.bool:
+                raise ValueError(f"request {r}: prompt must be a non-empty 1-D integer tensor")
+            if int(p.min()) < 0 or int(p.max()) >= V:
+                raise ValueError(f"request {r}: prompt tokens must lie in [0, {V})")
+            if int(q.gen_len) < 1:
+                raise ValueError(f"request {r}: gen_len must be >= 1, got {q.gen_len}")
+            if q.technique not in _TECHNIQUES:
+                raise ValueError(f"request {r}: unknown technique {q.technique!r} (one of {sorted(_TECHNIQUES)})")
+            if q.temperature < 0:
+                raise ValueError(f"request {r}: temperature must be >= 0")
+            prompts.append(p.tolist())
+            gen_lens.append(int(q.gen_len))
+            rows_i.append([_TECHNIQUES[q.technique], int(q.topk or 0), int(bool(q.exclude_bos)), int(q.empty_token),
+                           int(q.num_empty_tokens_to_ignore)])
+            rows_f.append([float(q.temperature), float(q.top_p)])
+        if uniforms is not None:
+            uniforms = list(uniforms)
+            if len(uniforms) != len(reqs):
+                raise ValueError(f"uniforms has {len(uniforms)} entries for {len(reqs)} requests")
+            for r, (u, g) in enumerate(zip(uniforms, gen_lens)):
+                if tuple(u.shape) != (g,):
+                    raise ValueError(f"uniforms[{r}] has shape {tuple(u.shape)}, expected ({g},)")
+        eng = self._get_engine()
+        dev = eng.device
+        sch = request_schedule(prompts, gen_lens, int(batch_size))
+        S, B = sch.tables.shape[1:]
+
+        def upload(t):  # pinned staging, one cudaMemcpyAsync: no synchronisation
+            return t.pin_memory().to(dev, non_blocking=True)
+
+        forced, req, out_off, key_start = upload(sch.tables)
+        req_i = upload(torch.tensor(rows_i, dtype=torch.int32))
+        req_f = upload(torch.tensor(rows_f, dtype=torch.float32))
+        u = None
+        if uniforms is not None:
+            us = [x.reshape(-1).float() for x in uniforms]
+            u = upload(torch.cat(us)) if all(x.device.type == "cpu" for x in us) else torch.cat([x.to(dev) for x in us])
+        out = torch.empty(sum(gen_lens), dtype=torch.int64, device=dev)
+        run = torch.zeros(B, dtype=torch.int32, device=dev)
+        cur = forced[0].to(torch.int64).view(1, B)  # the input tokens; tgan_sample_step writes the next ones in place
+        mems = eng.new_ring(B, 1, self.mem_len)  # empty, pos0 = 0: the row written at step t has position t
+        for t in range(S):
+            mems.key_start = key_start[t]  # a contiguous int32 row of the uploaded table: no copy
+            ectx = eng.forward(cur, None, mems, mem_len=self.mem_len, same_length=self.same_length, training=False,
+                               save_for_backward=False)
+            mems = ectx.new_mems
+            eng.calls += 1
+            L.sample_step(ectx.logits, req[t], key_start[t], out_off[t], forced[t + 1] if t + 1 < S else None, req_i,
+                          req_f, run, cur, out, V, t, u=u, seed=eng.seed, site=eng._site(eng.calls, 5))
+        return [out[b:b + g] for b, g in zip(sch.out_base, gen_lens)]

@@ -73,6 +73,7 @@ _SIGS = {
     "tgan_bert_attn_bwd": [I, P, L, P, L, P, P, L, I, I, I, I, F, U, U, P],
     "tgan_bert_attn_jvp": [I, P, L, P, L, P, P, L, I, I, I, I, F, U, U, P],
     "tgan_sample_tokens": [P, L, P, P, P, P, L, I, I, I, I, I, I, F, F, U, U, P],
+    "tgan_sample_step": [P, L, P, P, P, P, P, P, P, P, P, P, P, L, I, I, I, U, U, P],
     "tgan_nccl_load": [c_char_p],
     "tgan_nccl_unique_id": [P],
     "tgan_nccl_init": [P, I, I, P],
@@ -370,6 +371,17 @@ def sample_tokens(logits, ids, V, *, u=None, suppress_empty=None, probs_out=None
     _call("tgan_sample_tokens", logits.data_ptr(), logits.stride(0), _ptr(u), _ptr(suppress_empty), ids.data_ptr(),
           _ptr(probs_out), 0 if probs_out is None else probs_out.stride(0), rows, V, int(exclude_bos), empty_token, mode,
           topk, top_p, temperature, seed, site, _stream())
+
+
+def sample_step(logits, req, start, out_off, forced_next, req_i, req_f, run, cur, out, V, step, *, u=None,
+                probs_out=None, seed=0, site=0):
+    """One step of generation from a request queue (tgan_sample_step): logits fp32 [B, >= V]; req / start / out_off /
+    forced_next int32 [B] (forced_next may be None); req_i int32 [R, 5], req_f fp32 [R, 2]; run int32 [B] and cur int64
+    [B] are updated in place; out int64 / u fp32: flat buffers indexed by out_off."""
+    _call("tgan_sample_step", logits.data_ptr(), logits.stride(0), req.data_ptr(), start.data_ptr(), out_off.data_ptr(),
+          _ptr(forced_next), req_i.data_ptr(), req_f.data_ptr(), _ptr(u), run.data_ptr(), cur.data_ptr(),
+          out.data_ptr(), _ptr(probs_out), 0 if probs_out is None else probs_out.stride(0), req.numel(), V, step, seed,
+          site, _stream())
 
 
 def nccl_load(path=None):
