@@ -195,6 +195,18 @@ int tgan_colsum(int dtype, const void* x, int64_t ld, float* out, int rows, int 
  * Also the recurrence-memory import/export (mem_transformer.py:461-475): ring slab <-> reference fp32 mems. */
 int tgan_convert(int dtype_src, const void* src, int64_t lds, int dtype_dst, void* dst, int64_t ldd,
                  int64_t rows, int cols, int cols_pad, void* stream);
+/* Prefilled rows into a request queue's ring (generate.py:190-199's context pass, done once per group of prompts for
+ * MemTransformerLM.generate_requests): desc int32 [n][4] (16-byte aligned) = (source column, first source position,
+ * destination column, rows); descriptor i copies source positions [pos_i, pos_i + rows_i) of its column to destination
+ * positions [dst_end - rows_i, dst_end) of its column, in all n_slab layer-input slabs ([slab][pos][col][DP], slab
+ * strides src_x_stride / dst_x_stride elements) and all n_kv projected-K/V layers ([layer][pos][col][KW], strides
+ * src_kv_stride / dst_kv_stride; n_kv = 0: slabs only).  The source has src_cols columns, the destination dst_cols.
+ * dtype: F32 or BF16 on both sides; DP, KW multiples of 64, bases 16-byte aligned.  max_rows (>= every rows_i)
+ * sizes the grid only.  Descriptors must not overlap in the destination; rows_i = 0 copies nothing.          */
+int tgan_ring_scatter(int dtype, const int32_t* desc, int n, int max_rows, int dst_end, const void* src_x,
+                      int64_t src_x_stride, void* dst_x, int64_t dst_x_stride, int n_slab, int DP, const void* src_kv,
+                      int64_t src_kv_stride, void* dst_kv, int64_t dst_kv_stride, int n_kv, int KW, int src_cols,
+                      int dst_cols, void* stream);
 
 /* ---- parameter packing -----------------------------------------------------------------------------------
  * One launch converts the reference-layout fp32 parameters into the kernel-private padded layout, driven by a
@@ -256,7 +268,8 @@ int tgan_sample_tokens(const float* logits, int64_t ldl, const float* u, const u
  * serves request req[b] (-1 = idle), with that request's settings req_i int32 [R][5] = (mode, topk, exclude_bos,
  * empty_token, num_empty_tokens_to_ignore) and req_f fp32 [R][2] = (temperature, top_p), validated by the caller.
  * cur int64 [B] holds the column's input token of this step; run int32 [B] is the length of the run of empty_token
- * at the end of the column's inputs: reset where start[b] == step (a request starts), then extended by cur[b].  The
+ * at the end of the column's inputs: where start[b] == step (a request starts) it becomes run0[req[b]] (run0 int32
+ * [R], the run over the conditioning tokens a context pass consumed; NULL: 0), then it is extended by cur[b].  The
  * empty token is suppressed once run >= num_empty_tokens_to_ignore > 0.  The draw is tgan_sample_tokens' exact
  * arithmetic, on u[out_off[b]] (u != NULL and out_off[b] >= 0) or on Philox keyed by (seed, site, b).  The sample
  * goes to out[out_off[b]] when out_off[b] >= 0, and cur[b] becomes the next step's input: forced_next[b] when it
@@ -265,8 +278,8 @@ int tgan_sample_tokens(const float* logits, int64_t ldl, const float* u, const u
  * renormalised distribution of every busy column.                                                            */
 int tgan_sample_step(const float* logits, int64_t ldl, const int32_t* req, const int32_t* start,
                      const int32_t* out_off, const int32_t* forced_next, const int32_t* req_i, const float* req_f,
-                     const float* u, int32_t* run, int64_t* cur, int64_t* out, float* probs_out, int64_t ldp, int B,
-                     int V, int step, uint64_t seed, uint64_t site, void* stream);
+                     const float* u, const int32_t* run0, int32_t* run, int64_t* cur, int64_t* out, float* probs_out,
+                     int64_t ldp, int B, int V, int step, uint64_t seed, uint64_t site, void* stream);
 
 /* ---- data-parallel gradient all-reduce (SURVEY 8e): replaces DistributedDataParallel's implicit all-reduce,
  * train.py:649-655 / :904.  The library binds libnccl.so.2 at run time (tgan_nccl_load, optional explicit path).

@@ -15,3 +15,4 @@ run relattn tests/test_relattn_gpu.py
 run bert_attn tests/test_bert_attn_gpu.py
 run model tests/test_model_gpu.py
 run requests tests/test_generate_requests_gpu.py
+run requests_prefill tests/test_generate_requests_prefill_gpu.py

@@ -138,7 +138,7 @@ sample_kernel(const float* __restrict__ logits, int64_t ldl, const float* __rest
 // (-1 = idle) with that request's settings, sampled by the same row body as sample_kernel.
 struct StepArgs {
     const float* logits; int64_t ldl;
-    const int32_t *req, *start, *out_off, *forced_next, *req_i;
+    const int32_t *req, *start, *out_off, *forced_next, *req_i, *run0;
     const float *req_f, *u;
     int32_t* run; int64_t *cur, *out; float* probs_out; int64_t ldp;
     int B, V, step;
@@ -155,8 +155,9 @@ __global__ void __launch_bounds__(SW * 32) sample_step_kernel(StepArgs a) {
     if (r >= 0) {
         const int32_t* si = a.req_i + 5 * (int64_t)r;  // mode, topk, exclude_bos, empty_token, k
         const int empty_token = si[3], k = si[4];
-        // empty-bar run over the column's input tokens; a request starting at this step starts a new run
-        int run = a.start[b] == a.step ? 0 : a.run[b];
+        // empty-bar run over the column's input tokens; a request starting at this step starts a new run, from the run
+        // over the conditioning tokens its context pass consumed
+        int run = a.start[b] == a.step ? (a.run0 ? a.run0[r] : 0) : a.run[b];
         run = a.cur[b] == empty_token ? run + 1 : 0;
         const int off = a.out_off[b];
         const int token = sample_row(a.logits + (int64_t)b * a.ldl, s_p[warp], lane, a.V, k > 0 && run >= k, si[2],
@@ -197,15 +198,15 @@ extern "C" int tgan_sample_tokens(const float* logits, int64_t ldl, const float*
 
 extern "C" int tgan_sample_step(const float* logits, int64_t ldl, const int32_t* req, const int32_t* start,
                                 const int32_t* out_off, const int32_t* forced_next, const int32_t* req_i,
-                                const float* req_f, const float* u, int32_t* run, int64_t* cur, int64_t* out,
-                                float* probs_out, int64_t ldp, int B, int V, int step, uint64_t seed, uint64_t site,
-                                void* stream) {
+                                const float* req_f, const float* u, const int32_t* run0, int32_t* run, int64_t* cur,
+                                int64_t* out, float* probs_out, int64_t ldp, int B, int V, int step, uint64_t seed,
+                                uint64_t site, void* stream) {
     if (B <= 0) return 0;
     TGAN_CHECK_ARG(V >= 1 && V <= SMAXV, "tgan_sample_step: 1 <= V <= 1024");
     StepArgs a;
     a.logits = logits; a.ldl = ldl;
     a.req = req; a.start = start; a.out_off = out_off; a.forced_next = forced_next; a.req_i = req_i;
-    a.req_f = req_f; a.u = u;
+    a.req_f = req_f; a.u = u; a.run0 = run0;
     a.run = run; a.cur = cur; a.out = out; a.probs_out = probs_out; a.ldp = ldp;
     a.B = B; a.V = V; a.step = step; a.seed = seed; a.site = site;
     sample_step_kernel<<<ceil_div(B, SW), SW * 32, 0, (cudaStream_t)stream>>>(a);

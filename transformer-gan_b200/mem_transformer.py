@@ -12,7 +12,7 @@ import heapq
 import os
 import weakref
 from dataclasses import dataclass
-from typing import List, NamedTuple
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -248,6 +248,25 @@ class GenRequest:
     num_empty_tokens_to_ignore: int = 0
 
 
+class PrefillPlan(NamedTuple):
+    """The context passes of ``request_schedule(..., context_pass=True)``.  Requests are prefilled in groups of up to
+    ``batch_size`` consecutive requests (list order); group g's pass runs over ``blocks[g]`` (int64 [max(T_r - 1), G]:
+    column j holds prompt[:-1] of the group's j-th request, left-padded by ``pads[g][j]`` rows of token 0; None when
+    every prompt of the group is one token) and is enqueued at step ``steps[g]``, the start step of the group's first
+    request (None: no pass).  ``desc`` int32 [n, 4] lists, in request order, one (source column, first source position,
+    destination column, rows) copy per request with n_r = min(T_r - 1, mem_len) > 0 rows: the last n_r rows of its
+    pass.  ``slices[t]`` = [(group, first descriptor, count, max rows)] to apply at step t, in group order.
+    ``run0`` int32 [R]: the run of empty_token at the end of prompt[:-1].  ``lead`` = P0 = min(mem_len,
+    max_r(T_r - 1)): the queue ring's leading rows."""
+    lead: int
+    blocks: List[Optional[torch.Tensor]]
+    pads: List[torch.Tensor]
+    steps: List[Optional[int]]
+    desc: torch.Tensor
+    slices: Dict[int, List[Tuple[int, int, int, int]]]
+    run0: torch.Tensor
+
+
 class RequestSchedule(NamedTuple):
     """The step-by-column plan of ``generate_requests``.  ``tables`` int32 [4, S, B] holds, per step t and column b:
     forced   -- the input token of the step, or -1 for "the column's sample of step t - 1";
@@ -255,9 +274,13 @@ class RequestSchedule(NamedTuple):
     out_off  -- where the step's sample goes in the flat output, or -1 when it is not kept;
     key_start -- the step at which the column's current request started (an idle column: t itself).
     The row written at step t has absolute position t, so key_start is also the request's key floor.
-    ``out_base[r]``: offset of request r's first generated token in the flat output."""
+    ``out_base[r]``: offset of request r's first generated token in the flat output.
+    With a context pass (``prefill`` is not None) the tables are [5, S, B]: the row written at step t has absolute
+    position P0 + t, key_start is the key floor P0 + t0 - n_r of a request that starts at step t0 on its n_r prefilled
+    rows (an idle column: P0 + t), and the fifth row, ``start``, is the step at which the column's request started."""
     tables: torch.Tensor
     out_base: List[int]
+    prefill: Optional[PrefillPlan] = None
 
     @property
     def forced(self):
@@ -275,39 +298,101 @@ class RequestSchedule(NamedTuple):
     def key_start(self):
         return self.tables[3]
 
+    @property
+    def start(self):
+        return self.tables[4] if self.prefill is not None else self.tables[3]
 
-def request_schedule(prompts, gen_lens, batch_size) -> RequestSchedule:
+
+def _trailing_run(seq, token):
+    n = 0
+    for x in reversed(seq):
+        if x != token:
+            break
+        n += 1
+    return n
+
+
+def request_schedule(prompts, gen_lens, batch_size, *, context_pass=False, mem_len=None,
+                     empty_tokens=None) -> RequestSchedule:
     """Plan ``len(prompts)`` requests on min(batch_size, len(prompts)) columns.  Request r occupies one column for
     T_r + gen_len_r - 1 consecutive steps: it feeds its T_r prompt tokens one per step, the step that feeds the last
     one samples its first token, and each later step feeds the previous sample.  Requests go in list order to the
     column that frees first, ties to the lowest column.  Idle columns (the tail of the queue) are fed token 0 and floored
-    at their own row: they produce nothing.  prompts: 1-D int sequences (CPU); gen_lens: ints >= 1."""
+    at their own row: they produce nothing.  prompts: 1-D int sequences (CPU); gen_lens: ints >= 1.
+
+    context_pass=True: prompt[:-1] is consumed by context passes (``prefill``, see PrefillPlan) instead, so request r
+    occupies its column for gen_len_r steps only; its first step feeds prompt[-1] on its n_r = min(T_r - 1, mem_len)
+    prefilled rows.  Needs ``mem_len`` > 0; ``empty_tokens`` (one per request, default -1) sets ``run0``."""
+    if context_pass and not (mem_len or 0) > 0:
+        raise ValueError("a context pass needs mem_len > 0")
     B = min(batch_size, len(prompts))
+    R = len(prompts)
+    occupy = [g if context_pass else len(p) + g - 1 for p, g in zip(prompts, gen_lens)]
     free = [(0, c) for c in range(B)]  # (step at which the column frees, column): a heap
     place = []
-    for prompt, g in zip(prompts, gen_lens):
+    for n in occupy:
         t0, c = heapq.heappop(free)
         place.append((t0, c))
-        heapq.heappush(free, (t0 + len(prompt) + g - 1, c))
+        heapq.heappush(free, (t0 + n, c))
     S = max(t for t, _ in free)
-    tables = torch.empty(4, S, B, dtype=torch.int32)
-    forced, req, out_off, key_start = tables
+    tables = torch.empty(5 if context_pass else 4, S, B, dtype=torch.int32)
+    forced, req, out_off, key_start = tables[:4]
+    steps = torch.arange(S, dtype=torch.int32).view(S, 1).expand(S, B)
     forced.zero_()
     req.fill_(-1)
     out_off.fill_(-1)
-    key_start.copy_(torch.arange(S, dtype=torch.int32).view(S, 1).expand(S, B))
+    lead = min(mem_len, max(len(p) for p in prompts) - 1) if context_pass else 0
+    key_start.copy_(steps + lead)
+    if context_pass:
+        tables[4].copy_(steps)
     out_base, base = [], 0
-    for r, ((t0, c), prompt, g) in enumerate(zip(place, prompts, gen_lens)):
+    for r, ((t0, c), prompt, g, n) in enumerate(zip(place, prompts, gen_lens, occupy)):
         T = len(prompt)
-        n = T + g - 1
-        forced[t0:t0 + T, c] = torch.as_tensor(prompt, dtype=torch.int32)
-        forced[t0 + T:t0 + n, c] = -1
         req[t0:t0 + n, c] = r
-        out_off[t0 + T - 1:t0 + n, c] = torch.arange(base, base + g, dtype=torch.int32)
-        key_start[t0:t0 + n, c] = t0
+        if context_pass:
+            forced[t0, c] = int(prompt[-1])
+            forced[t0 + 1:t0 + n, c] = -1
+            out_off[t0:t0 + n, c] = torch.arange(base, base + g, dtype=torch.int32)
+            key_start[t0:t0 + n, c] = lead + t0 - min(T - 1, mem_len)
+            tables[4, t0:t0 + n, c] = t0
+        else:
+            forced[t0:t0 + T, c] = torch.as_tensor(prompt, dtype=torch.int32)
+            forced[t0 + T:t0 + n, c] = -1
+            out_off[t0 + T - 1:t0 + n, c] = torch.arange(base, base + g, dtype=torch.int32)
+            key_start[t0:t0 + n, c] = t0
         out_base.append(base)
         base += g
-    return RequestSchedule(tables, out_base)
+    if not context_pass:
+        return RequestSchedule(tables, out_base)
+    blocks, pads, pass_steps, desc, slices = [], [], [], [], {}
+    for gi, g0 in enumerate(range(0, R, B)):
+        members = range(g0, min(g0 + B, R))
+        Tm = max(len(prompts[r]) - 1 for r in members)
+        pad = torch.tensor([Tm - (len(prompts[r]) - 1) for r in members], dtype=torch.int32)
+        block = None
+        if Tm > 0:
+            block = torch.zeros(Tm, len(members), dtype=torch.int64)
+            for j, r in enumerate(members):
+                block[int(pad[j]):, j] = torch.as_tensor(prompts[r][:-1], dtype=torch.int64)
+        blocks.append(block)
+        pads.append(pad)
+        pass_steps.append(place[g0][0] if Tm > 0 else None)
+        for j, r in enumerate(members):
+            n_r = min(len(prompts[r]) - 1, mem_len)
+            if n_r == 0:
+                continue
+            t0, c = place[r]
+            sl = slices.setdefault(t0, [])
+            if sl and sl[-1][0] == gi:  # descriptors of one (group, step) are consecutive: request order
+                _, lo, cnt, mx = sl[-1]
+                sl[-1] = (gi, lo, cnt + 1, max(mx, n_r))
+            else:
+                sl.append((gi, len(desc), 1, n_r))
+            desc.append([j, Tm - n_r, c, n_r])
+    empty_tokens = [-1] * R if empty_tokens is None else list(empty_tokens)
+    run0 = torch.tensor([_trailing_run(list(p)[:-1], e) for p, e in zip(prompts, empty_tokens)], dtype=torch.int32)
+    plan = PrefillPlan(lead, blocks, pads, pass_steps, torch.tensor(desc, dtype=torch.int32).view(-1, 4), slices, run0)
+    return RequestSchedule(tables, out_base, plan)
 
 
 class MemTransformerLM(nn.Module):
@@ -583,23 +668,34 @@ class MemTransformerLM(nn.Module):
         return aligned, rows >= pad, ring
 
     @torch.no_grad()
-    def generate_requests(self, requests, batch_size, *, uniforms=None):
+    def generate_requests(self, requests, batch_size, *, uniforms=None, context_pass=False):
         """Continue every ``GenRequest`` of a queue, ``batch_size`` sequences at a time: a column that finishes a request
         takes the next one at the following step (``request_schedule``), so no column waits for the longest sequence
-        of a fixed batch.  Prompts are fed one token per step.  All columns share one ring memory; each column carries
-        a per-sequence key floor raised to the step at which its current request started, so a request never sees the
-        rows of the requests before it and computes what it computes alone.  Per step: the single-token forward of
-        ``generate_batched`` and one ``tgan_sample_step`` launch (per-request settings, empty-bar run, sampling, next
-        input), with no host synchronisation: the schedule is uploaded once, up front.
+        of a fixed batch.  All columns share one ring memory; each column carries a per-sequence key floor raised to
+        the first row of its current request, so a request never sees the rows of the requests before it and computes
+        what it computes alone.  Per step: the single-token forward of ``generate_batched`` and one
+        ``tgan_sample_step`` launch (per-request settings, empty-bar run, sampling, next input), with no host
+        synchronisation: the schedule is uploaded once, up front.
 
-        Request r's tokens equal ``generate_batched(prompt[:, None], gen_len, <its settings>, uniforms=u[:, None])``
-        up to rounding.  With ``same_length=False`` that holds for prompts of up to mem_len + 2 tokens: a longer prompt
-        row sees at most mem_len earlier rows here, as every single-token step does, while generate_batched's context
-        pass lets it see the whole prompt.
+        context_pass=False (the default): prompts are fed one token per step, so request r takes its column for
+        T_r + gen_len_r - 1 steps.  Request r's tokens equal ``generate_batched(prompt[:, None], gen_len, <its
+        settings>, uniforms=u[:, None])`` up to rounding; with ``same_length=False`` that holds for prompts of up to
+        mem_len + 2 tokens only: a longer prompt row sees at most mem_len earlier rows here, as every single-token step
+        does, while generate_batched's context pass lets it see the whole prompt.  The default keeps these semantics
+        for existing callers.
+
+        context_pass=True: prompt[:-1] of each group of ``batch_size`` consecutive requests goes through one ragged
+        context pass (the forward of ``generate_batched(prompt_lengths=)``); where a request starts, the last
+        min(T_r - 1, mem_len) rows of its pass (layer inputs and projected K/V) are copied into its column right below
+        the step's write position (``tgan_ring_scatter``), and the request takes its column for gen_len_r steps only.
+        Request r's tokens then equal ``generate_batched(prompt[:, None], gen_len, ...)`` alone up to rounding for every
+        prompt length and both ``same_length`` settings.
 
         requests: list of GenRequest.  uniforms: optional list with one [gen_len_r] tensor of uniforms in [0, 1) per
         request, replacing the device RNG (parity tests).  Returns a list whose entry r is request r's generated ids,
         int64 [gen_len_r] on the model's device (views into one buffer)."""
+        if not isinstance(context_pass, bool):
+            raise ValueError(f"context_pass must be a bool, got {context_pass!r}")
         reqs = list(requests)
         if not reqs:
             raise ValueError("generate_requests needs at least one request")
@@ -635,13 +731,16 @@ class MemTransformerLM(nn.Module):
                     raise ValueError(f"uniforms[{r}] has shape {tuple(u.shape)}, expected ({g},)")
         eng = self._get_engine()
         dev = eng.device
-        sch = request_schedule(prompts, gen_lens, int(batch_size))
+        sch = request_schedule(prompts, gen_lens, int(batch_size), context_pass=context_pass, mem_len=self.mem_len,
+                               empty_tokens=[row[3] for row in rows_i])
         S, B = sch.tables.shape[1:]
 
         def upload(t):  # pinned staging, one cudaMemcpyAsync: no synchronisation
             return t.pin_memory().to(dev, non_blocking=True)
 
-        forced, req, out_off, key_start = upload(sch.tables)
+        tables = upload(sch.tables)
+        forced, req, out_off, key_start = tables[:4]
+        start = tables[4] if context_pass else key_start
         req_i = upload(torch.tensor(rows_i, dtype=torch.int32))
         req_f = upload(torch.tensor(rows_f, dtype=torch.float32))
         u = None
@@ -651,13 +750,68 @@ class MemTransformerLM(nn.Module):
         out = torch.empty(sum(gen_lens), dtype=torch.int64, device=dev)
         run = torch.zeros(B, dtype=torch.int32, device=dev)
         cur = forced[0].to(torch.int64).view(1, B)  # the input tokens; tgan_sample_step writes the next ones in place
-        mems = eng.new_ring(B, 1, self.mem_len)  # empty, pos0 = 0: the row written at step t has position t
+        run0 = upload(sch.prefill.run0) if context_pass else None
+        for t, ectx in self._queue_forwards(eng, sch, key_start, cur, upload):
+            eng.calls += 1
+            L.sample_step(ectx.logits, req[t], start[t], out_off[t], forced[t + 1] if t + 1 < S else None, req_i,
+                          req_f, run, cur, out, V, t, u=u, run0=run0, seed=eng.seed, site=eng._site(eng.calls, 5))
+        return [out[b:b + g] for b, g in zip(sch.out_base, gen_lens)]
+
+    def _queue_forwards(self, eng, sch, key_start, cur, upload):
+        """The forwards of a request queue, one per step: yields (t, ctx of step t's single-token forward over ``cur``
+        [1, B]), the caller writing the next step's inputs into ``cur`` in between.  With a context pass, the prefill
+        passes and the copies of their rows run at their steps, before that step's forward.  key_start: the
+        schedule's key floors on the device; upload: host tensor -> device without synchronisation."""
+        S, B = sch.tables.shape[1:]
+        plan, events = sch.prefill, {}
+        if plan is not None:
+            desc = upload(plan.desc) if plan.desc.numel() else None
+            blocks = [b for b in plan.blocks if b is not None]
+            flat = upload(torch.cat([b.reshape(-1) for b in blocks])) if blocks else None
+            pads = upload(torch.cat(plan.pads))
+            passes, bo, po = [], 0, 0  # group g: (prompt block, pad) views into the uploads, or None
+            for b, pd in zip(plan.blocks, plan.pads):
+                passes.append(None if b is None else (flat[bo:bo + b.numel()].view(b.shape), pads[po:po + pd.numel()]))
+                bo += 0 if b is None else b.numel()
+                po += pd.numel()
+            # per step: the passes enqueued there and the copies applied there, a group's pass before its copies and
+            # the copies of an earlier group before a later group's pass (which releases the earlier prefill ring)
+            for g, t in enumerate(plan.steps):
+                if t is not None:
+                    events.setdefault(t, []).append((g, -1, 0, 0))
+            for t, sl in plan.slices.items():
+                events.setdefault(t, []).extend(sl)
+            for ev in events.values():
+                ev.sort()
+            last = {}  # group -> the step of its last copies, after which its prefill ring is released
+            for t, sl in plan.slices.items():
+                for g, *_ in sl:
+                    last[g] = max(last.get(g, t), t)
+            mems = eng.new_queue_ring(B, plan.lead, self.mem_len)  # the row written at step t has position P0 + t
+        else:
+            mems = eng.new_ring(B, 1, self.mem_len)  # empty, pos0 = 0: the row written at step t has position t
+        pre = None  # the ctx of the current group's prefill pass: the only reference to its ring
         for t in range(S):
+            for g, lo, n, max_rows in events.get(t, ()):
+                if lo < 0:
+                    pre = self._prefill_pass(eng, *passes[g])
+                else:
+                    mems = eng.scatter_prefill(mems, pre, desc, lo, n, max_rows, self.mem_len)
+                    if last[g] == t:
+                        pre = None  # every request of the group has its rows: release its prefill ring
             mems.key_start = key_start[t]  # a contiguous int32 row of the uploaded table: no copy
             ectx = eng.forward(cur, None, mems, mem_len=self.mem_len, same_length=self.same_length, training=False,
                                save_for_backward=False)
             mems = ectx.new_mems
-            eng.calls += 1
-            L.sample_step(ectx.logits, req[t], key_start[t], out_off[t], forced[t + 1] if t + 1 < S else None, req_i,
-                          req_f, run, cur, out, V, t, u=u, seed=eng.seed, site=eng._site(eng.calls, 5))
-        return [out[b:b + g] for b, g in zip(sch.out_base, gen_lens)]
+            yield t, ectx
+
+    def _prefill_pass(self, eng, blk, pad):
+        """One group's context pass over its prompt block blk (int64 [Tm, G], column j left-padded by pad[j] rows, pad
+        int32 [G]) into a ring of its own -> the forward's ctx (keep_kv=True), which scatter_prefill reads.  The pass
+        has no memory, so mem_len enters it only through the same_length shift, and that is the same for every
+        mem_len >= Tm: the ring is sized for min(mem_len, Tm) instead of the model's mem_len."""
+        ml = min(self.mem_len, blk.shape[0])
+        ring = eng.new_ring(blk.shape[1], blk.shape[0], ml)
+        ring.key_start = pad
+        return eng.forward(blk, None, ring, mem_len=ml, same_length=self.same_length, training=False,
+                           save_for_backward=False, keep_kv=True)

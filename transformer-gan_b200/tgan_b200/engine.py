@@ -493,12 +493,52 @@ class TxlEngine:
         new.key_start, new.pos0 = ring.key_start, ring.pos0  # logical row 0 stays row 0
         return new
 
+    def new_queue_ring(self, B: int, lead: int, mem_len: int) -> RingMems:
+        """The ring of a request queue whose prompts are prefilled by context passes (scatter_prefill): ``lead``
+        leading rows, zero and meant to be floored, then the decode steps' rows (pos0 = 0: the row of step t has
+        absolute position lead + t).  Its projected-K/V cache exists from the start, tagged with the current parameter
+        pack and covering the leading rows, so the first step projects only its new row and the K/V rows that
+        scatter_prefill writes count as cached."""
+        self.pack()
+        ring = self.new_ring(B, 1, mem_len)
+        ring.length = lead
+        buf = torch.empty(self.d.n_layer, ring.capacity, B, 2 * self.d.NH, dtype=self.dtype, device=self.device)
+        buf[:, :lead].zero_()
+        ring.kv.update(buf=buf, lo=0, hi=lead, tag=self.pack_epoch)
+        return ring
+
+    def scatter_prefill(self, ring: RingMems, src: _Ctx, desc: torch.Tensor, lo: int, n: int, max_rows: int,
+                        mem_len: int) -> RingMems:
+        """Copy prefilled rows into a request queue's ring right below the next single-token step's write position
+        (tgan_ring_scatter): descriptors desc[lo:lo+n] (device int32 [*, 4]: source column, first source position,
+        destination column, rows <= max_rows) read the ring and the K/V rows of ``src``, the ctx of a
+        ``forward(keep_kv=True)`` over the prompts.  The ring is prepared for that step first, so a re-layout that is
+        due happens before the copy and the rows land in the window the step reads.  Returns that ring."""
+        ring = self._prepare_ring(ring, ring.bsz, 1, mem_len)
+        w = ring.start + ring.length  # a decode ring keeps [memory; next row] contiguous: no wrap
+        if max_rows > ring.length:
+            raise L.TganError(f"internal: {max_rows} prefilled rows do not fit a window of {ring.length}")
+        st = ring.kv
+        kv_ok = st["buf"] is not None and st["tag"] == self.pack_epoch and st["lo"] <= ring.start and st["hi"] == w
+        kv, kv_stride = src.kv_rows
+        C, B = ring.capacity, ring.bsz
+        # a stale K/V cache is re-projected from the slabs by the next forward: then only the slabs are copied
+        L.ring_scatter(desc, n, max_rows, w, src.ring.slabs, ring.slabs, kv if kv_ok else None,
+                       st["buf"] if kv_ok else None, src_kv_stride=kv_stride, dst_kv_stride=C * B * 2 * self.d.NH,
+                       desc_off=lo)
+        return ring
+
     # -- forward ------------------------------------------------------------------------------------------
     def forward(self, inp: torch.Tensor, reset: Optional[torch.Tensor], mems, *, mem_len: int, same_length: bool,
                 training: bool, target: Optional[torch.Tensor] = None, n_pred: Optional[int] = None,
-                save_for_backward: bool = True) -> _Ctx:
+                save_for_backward: bool = True, keep_kv: bool = False) -> _Ctx:
         """inp: int64 [Q,B] token ids or float [Q,B,V] soft one-hot rows.  Returns a ctx with
-        ``nll`` (fp32 [T*B], when target is given), ``logits`` (fp32 [T*B, VP]) and ``new_mems``."""
+        ``nll`` (fp32 [T*B], when target is given), ``logits`` (fp32 [T*B, VP]) and ``new_mems``.
+        keep_kv: the ctx also exposes the projected K/V rows of every layer as ``kv_rows`` = (tensor, layer stride in
+        elements), row (position p, sequence b) of layer l at element l * stride + (p * B + b) * 2 * NH, p a physical
+        ring position (scatter_prefill reads them).  Calls with Q <= kv_cache_max_q find them in the ring's K/V cache;
+        longer ones keep their per-layer K/V rows in one [n_layer, K*B, 2*NH] buffer, which needs [memory; segment]
+        to start at ring position 0 (a fresh ring)."""
         d, lay, dt = self.d, self.layout, self.dtype
         DP, NH, DIP, VP, D = d.DP, d.NH, d.DIP, d.VP, d.d_model
         if save_for_backward and getattr(mems, "key_start", None) is not None:
@@ -538,6 +578,9 @@ class TxlEngine:
             else:
                 merged.append((pos, n))
         ctx.x_segs = merged
+        if keep_kv and not (Q <= self.kv_cache_max_q and mem_len > 0 and len(merged) == 1) and \
+                (len(merged) != 1 or merged[0][0] != 0):
+            raise L.TganError("keep_kv: a segment longer than kv_cache_max_q keeps its K/V rows only on a fresh ring")
         # same_length mask shift (mem_transformer.py:496-503)
         msl = Q
         if same_length:
@@ -581,6 +624,9 @@ class TxlEngine:
         # and only the new rows go through the GEMM.  Same values up to nothing: the rows are bit-identical.
         use_cache = Q <= self.kv_cache_max_q and mem_len > 0 and len(ctx.x_segs) == 1
         kv_from = 0
+        kv_all = None
+        if keep_kv and not use_cache:
+            kv_all = self._buf(d.n_layer, KR, 2 * NH)
         if use_cache:
             st, s0 = ring.kv, ctx.x_segs[0][0]
             if st["buf"] is None or st["buf"].shape[1:3] != (C, B) or st["buf"].dtype != dt:
@@ -612,7 +658,7 @@ class TxlEngine:
                 if side is not None:
                     main.wait_stream(side)
             else:
-                kv, kv_off = self._buf(KR, 2 * NH), 0
+                kv, kv_off = (self._buf(KR, 2 * NH) if kv_all is None else kv_all[l]), 0
                 row = 0
                 for pos, n in ctx.x_segs:
                     L.gemm(slabs, self.pmat, kv, M=n * B, N=2 * NH, K=DP, lda=DP, ldb=wld, a_off=x_base + pos * B * DP,
@@ -656,6 +702,8 @@ class TxlEngine:
             st = ring.kv
             st["lo"] = st["lo"] if kv_from == w and M > 0 else ctx.x_segs[0][0]
             st["hi"], st["tag"] = w + Q, self.pack_epoch
+        if keep_kv:
+            ctx.kv_rows = (ring.kv["buf"], C * B * 2 * NH) if use_cache else (kv_all, KR * 2 * NH)
         # 3. final dropout, logits, NLL
         T = Q if n_pred is None else n_pred
         ctx.T = T

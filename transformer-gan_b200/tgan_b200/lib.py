@@ -73,7 +73,8 @@ _SIGS = {
     "tgan_bert_attn_bwd": [I, P, L, P, L, P, P, L, I, I, I, I, F, U, U, P],
     "tgan_bert_attn_jvp": [I, P, L, P, L, P, P, L, I, I, I, I, F, U, U, P],
     "tgan_sample_tokens": [P, L, P, P, P, P, L, I, I, I, I, I, I, F, F, U, U, P],
-    "tgan_sample_step": [P, L, P, P, P, P, P, P, P, P, P, P, P, L, I, I, I, U, U, P],
+    "tgan_sample_step": [P, L, P, P, P, P, P, P, P, P, P, P, P, P, L, I, I, I, U, U, P],
+    "tgan_ring_scatter": [I, P, I, I, I, P, L, P, L, I, I, P, L, P, L, I, I, I, I, P],
     "tgan_nccl_load": [c_char_p],
     "tgan_nccl_unique_id": [P],
     "tgan_nccl_init": [P, I, I, P],
@@ -374,14 +375,32 @@ def sample_tokens(logits, ids, V, *, u=None, suppress_empty=None, probs_out=None
 
 
 def sample_step(logits, req, start, out_off, forced_next, req_i, req_f, run, cur, out, V, step, *, u=None,
-                probs_out=None, seed=0, site=0):
+                run0=None, probs_out=None, seed=0, site=0):
     """One step of generation from a request queue (tgan_sample_step): logits fp32 [B, >= V]; req / start / out_off /
     forced_next int32 [B] (forced_next may be None); req_i int32 [R, 5], req_f fp32 [R, 2]; run int32 [B] and cur int64
-    [B] are updated in place; out int64 / u fp32: flat buffers indexed by out_off."""
+    [B] are updated in place; out int64 / u fp32: flat buffers indexed by out_off; run0 (int32 [R] or None): the
+    empty-bar run a request starts with."""
     _call("tgan_sample_step", logits.data_ptr(), logits.stride(0), req.data_ptr(), start.data_ptr(), out_off.data_ptr(),
-          _ptr(forced_next), req_i.data_ptr(), req_f.data_ptr(), _ptr(u), run.data_ptr(), cur.data_ptr(),
+          _ptr(forced_next), req_i.data_ptr(), req_f.data_ptr(), _ptr(u), _ptr(run0), run.data_ptr(), cur.data_ptr(),
           out.data_ptr(), _ptr(probs_out), 0 if probs_out is None else probs_out.stride(0), req.numel(), V, step, seed,
           site, _stream())
+
+
+def ring_scatter(desc, n, max_rows, dst_end, src_x, dst_x, src_kv=None, dst_kv=None, *, src_kv_stride=0,
+                 dst_kv_stride=0, desc_off=0):
+    """tgan_ring_scatter: descriptors desc[desc_off : desc_off + n] (int32 [*, 4]: source column, first source position,
+    destination column, rows) copy rows of every slab of the ring slabs src_x [S, C, G, DP] into dst_x [S, C', B, DP],
+    landing at positions [dst_end - rows, dst_end); with src_kv / dst_kv also every layer of the projected-K/V rows
+    ([n_layer, *, G | B, KW] with layer strides src_kv_stride / dst_kv_stride elements, positions as in the slabs)."""
+    if src_x.dtype != dst_x.dtype or (src_kv is not None and (src_kv.dtype != src_x.dtype or dst_kv.dtype != src_x.dtype)):
+        raise TganError("ring_scatter: every buffer must have the same dtype")
+    if src_x.shape[0] != dst_x.shape[0] or src_x.shape[3] != dst_x.shape[3]:
+        raise TganError("ring_scatter: source and destination slabs differ in count or row width")
+    n_kv = 0 if src_kv is None else dst_kv.shape[0]
+    _call("tgan_ring_scatter", dtype_code(src_x.dtype), desc.data_ptr() + 16 * desc_off, n, max_rows, dst_end,
+          src_x.data_ptr(), src_x.stride(0), dst_x.data_ptr(), dst_x.stride(0), dst_x.shape[0], dst_x.shape[3],
+          _ptr(src_kv), src_kv_stride, _ptr(dst_kv), dst_kv_stride, n_kv, 0 if dst_kv is None else dst_kv.shape[-1],
+          src_x.shape[2], dst_x.shape[2], _stream())
 
 
 def nccl_load(path=None):
